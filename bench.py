@@ -7,7 +7,7 @@ Workload at N=1: BASELINE configs[1], 32 clips x 10 s (300 frames each, 9 600 fr
 N>1 each rank runs its own 32 clips (weak scaling, configs[4]); weights are broadcast from rank 0 once
 at load (NCCL) and there is no collective inside the step.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  `value` = device-timed frames/s with inputs resident in HBM; `e2e` = the
 same span through the public API with pinned HOST buffers (H2D audio + D2H results inside the timed
@@ -18,6 +18,11 @@ BASELINE configs (bs = 1 latency, CaMN bs 64, DisCo bs 32).
 `--impl reference` times the UNMODIFIED reference modules (byte-compiled into oracle/_ref by
 oracle/make_ref.py; falls back to the oracle port when that tree is absent) on the host cores, on the same
 32-clip step, same warm-up count.
+
+`--dump-outputs DIR` writes what the last device-timed step returned to its caller (rank 0) as DIR/<name>.npy, float32:
+the four SMPL-X outputs of decode() in full and the eight latents / logits of inference() on a fixed seeded sample of
+DUMP_LATENT_FRAMES frames (49.4 MB in all).  Weights and audio are seeded, so two builds run with the same arguments
+can be compared array by array.
 """
 from __future__ import annotations
 
@@ -49,6 +54,8 @@ NCU_TRAFFIC = {"bf16x6": (26.4e6, "profiles/ncu_full_r1_final.md"),
                "fp16x3": (8.711e6, "profiles/r2/ncu_full.md (8.711 MB read + 0 B written; algorithmic operand bytes 8.65 MB)")}
 METRIC = "motion_frames_per_sec"
 UNIT = "frames/s"
+DUMP_LATENT_FRAMES = 100              # of 300: keeps --dump-outputs under 64 MB
+DUMP_MAX_BYTES = 64 << 20
 
 
 def _peaks():
@@ -256,6 +263,25 @@ def _device_time(fn, steps, warmup, flush=None):
     return sum(s.elapsed_time(e) for s, e in ev) / steps
 
 
+def host_outputs(lat, pred):
+    """The (latent, pred) dicts a caller of the timed step receives, copied to host float32 arrays: pred in full, the
+    (clips, frames, 256) latents / logits on the same seeded frame sample in every run."""
+    import numpy as np
+    frames = np.sort(np.random.default_rng(0).choice(FRAMES_PER_CLIP, DUMP_LATENT_FRAMES, replace=False))
+    out = {k: v.float().cpu().numpy() for k, v in pred.items() if v is not None}
+    out.update({k: v[:, frames].float().cpu().numpy() for k, v in lat.items()})
+    return out
+
+
+def dump_outputs(out_dir, arrays):
+    import numpy as np
+    total = sum(v.nbytes for v in arrays.values())
+    assert total <= DUMP_MAX_BYTES, f"--dump-outputs would write {total} bytes"
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 def extra_configs(dev, peaks, flush, precision, cpu):
     """BASELINE configs[0] (one 10 s clip: latency, weight-bandwidth bound), [2] CaMN bs 64, [3] DisCo bs 32."""
     import torch
@@ -364,8 +390,8 @@ def run_gpu(args):
         if cap is not None:
             cap.graph.replay()
             ops.launch_count += cap.kernels_per_replay
-        else:
-            generate(model, vqm, audio)
+            return cap.latent, cap.pred
+        return generate(model, vqm, audio)
 
     def step_e2e():
         if cap is not None:
@@ -374,7 +400,7 @@ def run_gpu(args):
 
     warmup = max(args.warmup, 3)
     for _ in range(warmup):
-        step_resident()
+        last = step_resident()             # held like in the timed loop, so the allocator has warmed up for it
     sync_all()
 
     sampler = ClockSampler(local)
@@ -388,11 +414,14 @@ def run_gpu(args):
     for i in range(args.steps):
         flush.fill_(i & 0xFF)                   # evict L2 between timed iterations (outside the bracket)
         starts[i].record()
-        step_resident()
+        last = step_resident()
         ends[i].record()
     sync_all()
     launches = ops.launch_count - launches0
     dev_ms = sum(s.elapsed_time(e) for s, e in zip(starts, ends))
+    # copied now: the e2e steps below replay the same graph into the same output tensors
+    dumped = host_outputs(*last) if args.dump_outputs and rank == 0 else None
+    del last
 
     # ---- e2e: pinned host audio -> H2D -> public API -> D2H of the emitted SMPL-X parameters ----
     out_host = {k: torch.empty(clips, FRAMES_PER_CLIP, d).pin_memory() for k, d in
@@ -476,6 +505,8 @@ def run_gpu(args):
             "extra": extra,
             "clocks": clocks,
         }
+        if dumped is not None:
+            dump_outputs(args.dump_outputs, dumped)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()
@@ -494,7 +525,13 @@ def main():
     ap.add_argument("--extra", type=int, default=1, help="0 skips the other BASELINE configs (bs 1, CaMN, DisCo)")
     ap.add_argument("--body-priority", type=int, default=1, help="capture the critical (body) chain on a high-priority stream")
     ap.add_argument("--graph", type=int, default=1, help="replay the step as one CUDA graph (1) or launch eagerly (0)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (GPU arm only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU arm's outputs; it does not apply to --impl reference")
     if args.impl == "reference":
         run_reference(args)
     else:
