@@ -178,6 +178,61 @@ int pm_pose_compose_f32(const float* face, const float* upper, const float* hand
 int pm_global_trans_f32(const float* rec, int ld, int vel_off, const float* ref_trans, int ref_bs, float dt,
                         float* trans, int batch, int t, void* stream);
 
+/* ---- ragged batches: clips of different lengths laid out at one capacity ----------------------------------------
+ * Each entry point below is the one of the same name without `_rl`, plus per-clip limits, and runs the same kernel
+ * (a NULL limit is that entry point).  They keep one invariant, which makes a clip's result in a ragged batch equal
+ * its result alone: no kernel that mixes rows (convolution, attention) ever reads a padded row as data.  Limit
+ * tables are DEVICE int32 arrays, so a captured graph reads whatever the caller copied into them before a replay.
+ *   pm_tapgemm_tc_rl / pm_tapgemm_f32_rl  output row r of clip c is computed as usual if r < row_limit[c]; otherwise
+ *       its fp32 and plane outputs are stored as 0 (bias and residual are not read) - the zero padding the next
+ *       convolution expects - and a NEGATIVE limit leaves all rows of the clip unwritten.  The clip of output row
+ *       (b, l) is b when rows_per_clip == 0, else (b*rows_out + l) / rows_per_clip with row r = the remainder (a
+ *       Linear over all clips as one tall matrix).
+ *   pm_wav_stem_rl       sequence s (window-major, w*batch + b) holds n_valid[s] <= n_samples samples: later samples
+ *       read as 0 (the right-hand zero padding) and rows >= (n_valid + 2*pad - ksize)/stride + 1 are written as 0
+ *       (all rows for n_valid == 0).
+ *   pm_attention_tc_rl / pm_attention_f32_rl  keys >= k_len[b] get probability 0; query rows >= q_len[b] are written as
+ *       0, and so is every row of a clip with k_len[b] == 0.
+ *   pm_window_input_rl   rows >= win_len_valid[b] are written as 0.
+ *   pm_gather_rows_rl    row r belongs to clip r / rows_per_clip (> 0); rows with r % rows_per_clip >= row_limit[clip]
+ *       are written as 0. */
+int pm_tapgemm_tc_rl(const uint16_t* A, long long a_ps, long long a_bs, int lda, int batch, int rows_in, int cin,
+                     const uint16_t* W, long long w_ps, int w_rows, int ldw, int taps, int pad, int nsplit,
+                     const float* bias, int rows_out, int cout,
+                     const float* residual, long long r_bs, int ldr,
+                     int act, int act_cols, float slope, float acc_scale,
+                     float* out_f32, long long o_bs, int ldo,
+                     uint16_t* out_bf16, long long ob_ps, long long ob_bs, int ldob, int out_nsplit,
+                     const void* prefetch, long long prefetch_bytes, const int* row_limit, int rows_per_clip,
+                     void* stream);
+int pm_tapgemm_f32_rl(const float* A, long long a_bs, int lda, int batch, int rows_in, int cin,
+                      const float* W, const float* bias, int taps, int stride, int pad,
+                      int rows_out, int cout,
+                      const float* residual, long long r_bs, int ldr,
+                      int act, float slope,
+                      float* out, long long o_bs, int ldo, const int* row_limit, int rows_per_clip, void* stream);
+int pm_wav_stem_rl(const float* audio, long long a_bs, long long a_ws, int batch, int windows, int n_samples,
+                   const float* w1, const float* b1, const float* wd, const float* bd, int cout,
+                   int ksize, int stride, int pad, int rows_out, float slope,
+                   float* y1, float* sc,
+                   uint16_t* planes, long long p_ps, int p_ld, int p_nsplit, const int* n_valid, void* stream);
+int pm_attention_tc_rl(const uint16_t* Q, long long q_ps, long long q_bs, int ldq, int q_cols, int q_col0,
+                       const uint16_t* K, long long k_ps, long long k_bs, int ldk, int k_cols, int k_col0,
+                       const uint16_t* V, long long v_ps, long long v_bs, int ldv, int v_cols, int v_col0,
+                       float* O, int ldo, int batch, int heads, int tq, int tk, int head_dim,
+                       uint16_t* planes, long long p_ps, int p_ld, int p_nsplit, const int* q_len, const int* k_len,
+                       void* stream);
+int pm_attention_f32_rl(const float* Q, int ldq, const float* K, int ldk, const float* V, int ldv,
+                        float* O, int ldo, int batch, int heads, int tq, int tk, int head_dim,
+                        uint16_t* planes, long long p_ps, int p_ld, int p_nsplit, const int* q_len, const int* k_len,
+                        void* stream);
+int pm_window_input_rl(const float* motion, const float* mask, const float* seed, const float* mask_embedding,
+                       float* out, int batch, int total_len, int start, int win_len, int pre, int ch, long long seed_bs,
+                       uint16_t* planes, long long p_ps, int p_ld, int p_nsplit, const int* win_len_valid, void* stream);
+int pm_gather_rows_rl(const float* codebook, long long n_table, const long long* index, long long rows, int ch,
+                      float* out, uint16_t* planes, long long p_ps, int p_ld, int p_nsplit,
+                      const int* row_limit, int rows_per_clip, void* stream);
+
 /* ---- CaMN / DisCo (BASELINE configs[2],[3]) ------------------------------------------------------- */
 /* One bidirectional nn.LSTM layer, zero initial state (camn:205-217,264-271; disco:212-216,255).  xproj (batch, t,
  * ldx >= 8*hidden) holds W_ih x + b_ih + b_hh for both directions (column dir*4H + gate*H + unit, gates i,f,g,o);

@@ -45,6 +45,13 @@ SIGNATURES = {
     "pm_rot6d_to_aa_f32": [_p, _ll, _i, _p, _p, _p],
     "pm_softmax2_mix_f32": [_p, _p, _p, _p, _ll, _i, _i, _p],
 }
+# ragged-batch twins: the entry point without `_rl` + per-clip limit arguments before the stream
+for _rl, _name, _extra in (("pm_tapgemm_tc_rl", "pm_tapgemm_tc", [_p, _i]), ("pm_tapgemm_f32_rl", "pm_tapgemm_f32", [_p, _i]),
+                           ("pm_wav_stem_rl", "pm_wav_stem_f32", [_p]), ("pm_attention_tc_rl", "pm_attention_tc", [_p, _p]),
+                           ("pm_attention_f32_rl", "pm_attention_f32", [_p, _p]),
+                           ("pm_window_input_rl", "pm_window_input_f32", [_p]),
+                           ("pm_gather_rows_rl", "pm_gather_rows_f32", [_p, _i])):
+    SIGNATURES[_rl] = SIGNATURES[_name][:-1] + _extra + [_p]
 
 _lib = None
 

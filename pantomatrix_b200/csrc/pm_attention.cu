@@ -18,7 +18,7 @@ template <bool F16>
 __global__ void __launch_bounds__(NT) attention_f32_kernel(
     const float* __restrict__ Q, int ldq, const float* __restrict__ K, int ldk,
     const float* __restrict__ V, int ldv, float* __restrict__ O, int ldo,
-    int heads, int tq, int tk, float scale, PmPlanes P) {
+    int heads, int tq, int tk, float scale, PmPlanes P, const int* __restrict__ q_len, const int* __restrict__ k_len) {
   extern __shared__ float smem[];
   float* Qs = smem;                    // [TMAX][HDP]
   float* Ks = Qs + TMAX * HDP;         // [TMAX][HDP]
@@ -26,6 +26,10 @@ __global__ void __launch_bounds__(NT) attention_f32_kernel(
   float* S = Vs + TMAX * HD;           // [TMAX][TMAX+1]
   const int b = blockIdx.x / heads, h = blockIdx.x % heads;
   const int tid = threadIdx.x;
+  // ragged batches (pm_attention_f32_rl): keys beyond the clip's count get probability 0, query rows beyond its count
+  // (every row when it has no key) are written as 0
+  const int tkv = k_len ? min(tk, __ldg(k_len + b)) : tk;
+  const int tqv = q_len ? min(tq, __ldg(q_len + b)) : tq;
 
   // stage Q, K, V head slices (float4 global loads, scalar smem stores because of the +1 padding)
   for (int i = tid; i < TMAX * (HD / 4); i += NT) {
@@ -76,11 +80,11 @@ __global__ void __launch_bounds__(NT) attention_f32_kernel(
     const int warp = tid >> 5, lane = tid & 31;
     for (int r = warp; r < tq; r += NT / 32) {
       float* row = S + r * (TMAX + 1);
-      const float v0 = lane < tk ? row[lane] : -INFINITY;
-      const float v1 = lane + 32 < tk ? row[lane + 32] : -INFINITY;
+      const float v0 = lane < tkv ? row[lane] : -INFINITY;
+      const float v1 = lane + 32 < tkv ? row[lane + 32] : -INFINITY;
       const float m = pm_warp_max(fmaxf(v0, v1));
-      const float e0 = lane < tk ? expf(v0 - m) : 0.f;
-      const float e1 = lane + 32 < tk ? expf(v1 - m) : 0.f;
+      const float e0 = lane < tkv ? expf(v0 - m) : 0.f;
+      const float e1 = lane + 32 < tkv ? expf(v1 - m) : 0.f;
       const float inv = 1.f / pm_warp_sum(e0 + e1);
       row[lane] = e0 * inv;
       row[lane + 32] = e1 * inv;
@@ -96,7 +100,7 @@ __global__ void __launch_bounds__(NT) attention_f32_kernel(
     for (int a = 0; a < 4; ++a)
 #pragma unroll
       for (int m = 0; m < 12; ++m) acc[a][m] = 0.f;
-    for (int j = 0; j < tk; ++j) {
+    for (int j = 0; j < tkv; ++j) {
       float pv[4];
 #pragma unroll
       for (int a = 0; a < 4; ++a) pv[a] = S[(tr * 4 + a) * (TMAX + 1) + j];
@@ -121,7 +125,8 @@ __global__ void __launch_bounds__(NT) attention_f32_kernel(
     const bool vec_p = P.ptr && ((P.ld & 3) == 0) && ((P.ps & 3) == 0) && ((reinterpret_cast<uintptr_t>(P.ptr) & 7) == 0);
     for (int i = tid; i < tq * (HD / 4); i += NT) {
       const int r = i / (HD / 4), c4 = i % (HD / 4);
-      const float4 v = *reinterpret_cast<const float4*>(Os + r * HD + c4 * 4);
+      const float4 v = (r < tqv && tkv > 0) ? *reinterpret_cast<const float4*>(Os + r * HD + c4 * 4)
+                                             : make_float4(0.f, 0.f, 0.f, 0.f);
       const long long row = (long long)b * tq + r;
       if (O) *reinterpret_cast<float4*>(O + row * ldo + h * HD + c4 * 4) = v;
       if (P.ptr) {
@@ -139,9 +144,10 @@ constexpr size_t kSmemBytes = (size_t)(2 * TMAX * HDP + TMAX * HD + TMAX * (TMAX
 
 }  // namespace
 
-extern "C" int pm_attention_f32(const float* Q, int ldq, const float* K, int ldk, const float* V, int ldv,
-                                float* O, int ldo, int batch, int heads, int tq, int tk, int head_dim,
-                                uint16_t* planes, long long p_ps, int p_ld, int p_nsplit, void* stream) {
+static int attention_f32_run(const float* Q, int ldq, const float* K, int ldk, const float* V, int ldv,
+                             float* O, int ldo, int batch, int heads, int tq, int tk, int head_dim,
+                             uint16_t* planes, long long p_ps, int p_ld, int p_nsplit, const int* q_len, const int* k_len,
+                             void* stream) {
   PM_REQUIRE(Q && K && V && (O || planes) && batch >= 0 && heads > 0);
   PM_TAKE_FMT(p_nsplit, f16);
   PM_REQUIRE(pm_planes_ok(planes, p_ps, p_ld, p_nsplit, heads * head_dim, false));
@@ -158,8 +164,23 @@ extern "C" int pm_attention_f32(const float* Q, int ldq, const float* K, int ldk
     if (e != cudaSuccess) { configured = 0; return (int)e; }
   }
   if (f16) attention_f32_kernel<true><<<batch * heads, NT, kSmemBytes, (cudaStream_t)stream>>>(
-      Q, ldq, K, ldk, V, ldv, O, ldo, heads, tq, tk, 1.0f / sqrtf((float)head_dim), P);
+      Q, ldq, K, ldk, V, ldv, O, ldo, heads, tq, tk, 1.0f / sqrtf((float)head_dim), P, q_len, k_len);
   else attention_f32_kernel<false><<<batch * heads, NT, kSmemBytes, (cudaStream_t)stream>>>(
-      Q, ldq, K, ldk, V, ldv, O, ldo, heads, tq, tk, 1.0f / sqrtf((float)head_dim), P);
+      Q, ldq, K, ldk, V, ldv, O, ldo, heads, tq, tk, 1.0f / sqrtf((float)head_dim), P, q_len, k_len);
   PM_LAUNCH_CHECK();
+}
+
+extern "C" int pm_attention_f32(const float* Q, int ldq, const float* K, int ldk, const float* V, int ldv,
+                                float* O, int ldo, int batch, int heads, int tq, int tk, int head_dim,
+                                uint16_t* planes, long long p_ps, int p_ld, int p_nsplit, void* stream) {
+  return attention_f32_run(Q, ldq, K, ldk, V, ldv, O, ldo, batch, heads, tq, tk, head_dim, planes, p_ps, p_ld, p_nsplit,
+                           nullptr, nullptr, stream);
+}
+
+extern "C" int pm_attention_f32_rl(const float* Q, int ldq, const float* K, int ldk, const float* V, int ldv,
+                                   float* O, int ldo, int batch, int heads, int tq, int tk, int head_dim,
+                                   uint16_t* planes, long long p_ps, int p_ld, int p_nsplit, const int* q_len,
+                                   const int* k_len, void* stream) {
+  return attention_f32_run(Q, ldq, K, ldk, V, ldv, O, ldo, batch, heads, tq, tk, head_dim, planes, p_ps, p_ld, p_nsplit,
+                           q_len, k_len, stream);
 }

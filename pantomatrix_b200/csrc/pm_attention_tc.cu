@@ -50,6 +50,7 @@ struct AttnParams {
   float scale;                          // 1 / (sqrt(hd) * 64 * 64): the operand planes hold 64 x
   float* out; int ldo;                  // fp32 (batch*tq, >= heads*hd) or null
   PmPlanes planes;                      // fp16 planes of the output or ptr == null
+  const int* q_len; const int* k_len;   // ragged batches (pm_attention_tc_rl, nullable): per-clip query / key counts
 };
 
 __device__ __forceinline__ void tmem_ld64(uint32_t taddr, uint32_t (&r)[64]) {
@@ -179,10 +180,11 @@ __global__ void __launch_bounds__(NTHREADS, 1) attention_tc_kernel(const __grid_
       // (2 ulp); expf() costs ~25 instructions per element on 16 active lanes - the softmax was 5 400 of the kernel's
       // 20 000 cycles (profiles/r2/attention_timeline.md)
       const float sl2 = p.scale * 1.4426950408889634f;
+      const int tk = p.k_len ? min(p.tk, __ldg(p.k_len + b)) : p.tk;      // keys beyond a clip's count: probability 0
       float m = -INFINITY;
 #pragma unroll
       for (int j = 0; j < 64; ++j) {
-        const float v = j < p.tk ? __uint_as_float(sr[j]) * sl2 : -INFINITY;
+        const float v = j < tk ? __uint_as_float(sr[j]) * sl2 : -INFINITY;
         sr[j] = __float_as_uint(v);
         m = fmaxf(m, v);
       }
@@ -190,11 +192,11 @@ __global__ void __launch_bounds__(NTHREADS, 1) attention_tc_kernel(const __grid_
 #pragma unroll
       for (int j = 0; j < 64; ++j) {
         float e = 0.f;
-        if (j < p.tk) asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e) : "f"(__uint_as_float(sr[j]) - m));
+        if (j < tk) asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e) : "f"(__uint_as_float(sr[j]) - m));
         sum += e;
         sr[j] = __float_as_uint(e * P_SCALE);
       }
-      inv = 1.f / (sum * (P_SCALE * PM_F16_ACT_SCALE));
+      inv = tk > 0 ? 1.f / (sum * (P_SCALE * PM_F16_ACT_SCALE)) : 0.f;
       if (active) {
         const uint32_t dst = sm_u + Smem::P + (row >> 3) * 1024 + (row & 7) * 128;
 #pragma unroll
@@ -226,6 +228,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) attention_tc_kernel(const __grid_
     tc_fence_after();
     if (warp == 0) AT_STAMP(4);                            // O complete
     const bool live = active && row < p.tq;
+    // ragged batches: query rows beyond the clip's count (and every row of a clip without keys) are written as 0
+    const bool zero = (p.q_len && row >= __ldg(p.q_len + b)) || (p.k_len && __ldg(p.k_len + b) <= 0);
     const long long grow = (long long)b * p.tq + row;
     const bool vec16 = p.planes.ptr && ((p.planes.ld & 7) == 0) && ((p.planes.ps & 7) == 0) &&
                        ((reinterpret_cast<uintptr_t>(p.planes.ptr) & 15) == 0);
@@ -240,7 +244,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) attention_tc_kernel(const __grid_
         for (int g8 = 0; g8 < 8; ++g8) {                   // 8 consecutive columns
           float x[8];
 #pragma unroll
-          for (int u = 0; u < 8; ++u) x[u] = __uint_as_float(orr[8 * g8 + u]) * inv;
+          for (int u = 0; u < 8; ++u) x[u] = zero ? 0.f : __uint_as_float(orr[8 * g8 + u]) * inv;
           if (frow) {
             *reinterpret_cast<float4*>(frow + c0 + 8 * g8) = make_float4(x[0], x[1], x[2], x[3]);
             *reinterpret_cast<float4*>(frow + c0 + 8 * g8 + 4) = make_float4(x[4], x[5], x[6], x[7]);
@@ -292,11 +296,12 @@ bool plane_map(CUtensorMap* m, const uint16_t* base, long long ps, long long bs,
 
 }  // namespace
 
-extern "C" int pm_attention_tc(const uint16_t* Q, long long q_ps, long long q_bs, int ldq, int q_cols, int q_col0,
-                               const uint16_t* K, long long k_ps, long long k_bs, int ldk, int k_cols, int k_col0,
-                               const uint16_t* V, long long v_ps, long long v_bs, int ldv, int v_cols, int v_col0,
-                               float* O, int ldo, int batch, int heads, int tq, int tk, int head_dim,
-                               uint16_t* planes, long long p_ps, int p_ld, int p_nsplit, void* stream) {
+static int attention_tc_run(const uint16_t* Q, long long q_ps, long long q_bs, int ldq, int q_cols, int q_col0,
+                            const uint16_t* K, long long k_ps, long long k_bs, int ldk, int k_cols, int k_col0,
+                            const uint16_t* V, long long v_ps, long long v_bs, int ldv, int v_cols, int v_col0,
+                            float* O, int ldo, int batch, int heads, int tq, int tk, int head_dim,
+                            uint16_t* planes, long long p_ps, int p_ld, int p_nsplit, const int* q_len, const int* k_len,
+                            void* stream) {
   PM_REQUIRE(Q && K && V && (O || planes) && batch >= 0 && heads > 0);
   PM_TAKE_FMT(p_nsplit, f16);
   PM_REQUIRE(!planes || (f16 && p_nsplit <= 2));           // fp16 planes in, (at most two) fp16 planes out
@@ -319,6 +324,7 @@ extern "C" int pm_attention_tc(const uint16_t* Q, long long q_ps, long long q_bs
   p.scale = 1.0f / (sqrtf((float)head_dim) * PM_F16_ACT_SCALE * PM_F16_ACT_SCALE);
   p.out = O; p.ldo = ldo;
   p.planes = PmPlanes{reinterpret_cast<__nv_bfloat16*>(planes), p_ps, p_ld, p_nsplit};
+  p.q_len = q_len; p.k_len = k_len;
   static unsigned long long configured = 0;
   if (pm_first_use_on_device(configured)) {
     cudaError_t e = cudaFuncSetAttribute(attention_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmem);
@@ -326,6 +332,27 @@ extern "C" int pm_attention_tc(const uint16_t* Q, long long q_ps, long long q_bs
   }
   attention_tc_kernel<<<batch * heads, NTHREADS, kSmem, (cudaStream_t)stream>>>(mq, mk, mv, p);
   PM_LAUNCH_CHECK();
+}
+
+extern "C" int pm_attention_tc(const uint16_t* Q, long long q_ps, long long q_bs, int ldq, int q_cols, int q_col0,
+                               const uint16_t* K, long long k_ps, long long k_bs, int ldk, int k_cols, int k_col0,
+                               const uint16_t* V, long long v_ps, long long v_bs, int ldv, int v_cols, int v_col0,
+                               float* O, int ldo, int batch, int heads, int tq, int tk, int head_dim,
+                               uint16_t* planes, long long p_ps, int p_ld, int p_nsplit, void* stream) {
+  return attention_tc_run(Q, q_ps, q_bs, ldq, q_cols, q_col0, K, k_ps, k_bs, ldk, k_cols, k_col0, V, v_ps, v_bs, ldv,
+                          v_cols, v_col0, O, ldo, batch, heads, tq, tk, head_dim, planes, p_ps, p_ld, p_nsplit, nullptr,
+                          nullptr, stream);
+}
+
+extern "C" int pm_attention_tc_rl(const uint16_t* Q, long long q_ps, long long q_bs, int ldq, int q_cols, int q_col0,
+                                  const uint16_t* K, long long k_ps, long long k_bs, int ldk, int k_cols, int k_col0,
+                                  const uint16_t* V, long long v_ps, long long v_bs, int ldv, int v_cols, int v_col0,
+                                  float* O, int ldo, int batch, int heads, int tq, int tk, int head_dim,
+                                  uint16_t* planes, long long p_ps, int p_ld, int p_nsplit, const int* q_len,
+                                  const int* k_len, void* stream) {
+  return attention_tc_run(Q, q_ps, q_bs, ldq, q_cols, q_col0, K, k_ps, k_bs, ldk, k_cols, k_col0, V, v_ps, v_bs, ldv,
+                          v_cols, v_col0, O, ldo, batch, heads, tq, tk, head_dim, planes, p_ps, p_ld, p_nsplit, q_len,
+                          k_len, stream);
 }
 
 #ifdef PM_ATTN_TIMING

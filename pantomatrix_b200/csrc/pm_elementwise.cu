@@ -39,7 +39,7 @@ __global__ void __launch_bounds__(STEM_THREADS, 2) wav_stem_kernel(
     const float* __restrict__ audio, long long a_bs, long long a_ws, int batch, int n_samples,
     const float* __restrict__ w1, const float* __restrict__ b1, const float* __restrict__ wd,
     const float* __restrict__ bd, int stride, int pad, int rows_out, float slope,
-    float* __restrict__ y1, float* __restrict__ sc, const PmPlanes P) {
+    float* __restrict__ y1, float* __restrict__ sc, const PmPlanes P, const int* __restrict__ n_valid) {
   extern __shared__ float sx[];            // the input span of this tile: (STEM_ROWS - 1) * stride + KS samples
   constexpr int LPR = COUT / 2;            // lanes per row (a lane owns channels 2*cp, 2*cp + 1)
   constexpr int RW = 32 / LPR;             // row groups per warp
@@ -50,9 +50,17 @@ __global__ void __launch_bounds__(STEM_THREADS, 2) wav_stem_kernel(
   const float* __restrict__ x = audio + (long long)b * a_bs + (long long)w * a_ws;
   const int l0 = blockIdx.x * STEM_ROWS;
   const int span = (STEM_ROWS - 1) * stride + KS;
+  // ragged batches: the slice holds n_valid[seq] samples (the rest reads as the reference's zero padding) and only
+  // the rows the shorter slice yields are valid; the others are written as 0 for the convolutions that follow
+  int n_in = n_samples, valid_rows = rows_out;
+  if (n_valid) {
+    n_in = min(n_samples, __ldg(n_valid + seq));
+    const int num = n_in + 2 * pad - KS;
+    valid_rows = n_in <= 0 || num < 0 ? 0 : min(rows_out, num / stride + 1);
+  }
   for (int i = threadIdx.x; i < span; i += STEM_THREADS) {
     const int s = l0 * stride - pad + i;
-    sx[i] = (s >= 0 && s < n_samples) ? x[s] : 0.f;
+    sx[i] = (s >= 0 && s < n_in) ? x[s] : 0.f;
   }
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int cp = lane % LPR, rs = lane / LPR;
@@ -110,8 +118,10 @@ __global__ void __launch_bounds__(STEM_THREADS, 2) wav_stem_kernel(
       float a0 = acc[j][0] + ba0, a1 = acc[j][1] + ba1;
       a0 = a0 > 0.f ? a0 : a0 * slope;
       a1 = a1 > 0.f ? a1 : a1 * slope;
+      float s0 = acc[j][2] + bb0, s1 = acc[j][3] + bb1;
+      if (l >= valid_rows) a0 = a1 = s0 = s1 = 0.f;
       const long long row = (long long)seq * rows_out + l;
-      *reinterpret_cast<float2*>(sc + row * COUT + c0) = make_float2(acc[j][2] + bb0, acc[j][3] + bb1);
+      *reinterpret_cast<float2*>(sc + row * COUT + c0) = make_float2(s0, s1);
       if (y1) *reinterpret_cast<float2*>(y1 + row * COUT + c0) = make_float2(a0, a1);
       if (P.ptr) stem_store_planes2<F16>(P, row, c0, a0, a1);
     }
@@ -220,7 +230,8 @@ template <bool F16>
 __global__ void __launch_bounds__(256) window_input_kernel(
     const float* __restrict__ motion, const float* __restrict__ mask, const float* __restrict__ seed,
     const float* __restrict__ mask_embedding, float* __restrict__ out,
-    int batch, int total_len, int start, int win_len, int pre, int ch, long long seed_bs, PmPlanes P) {
+    int batch, int total_len, int start, int win_len, int pre, int ch, long long seed_bs, PmPlanes P,
+    const int* __restrict__ win_len_valid) {
   const long long total = (long long)batch * win_len * ch;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total;
        i += (long long)gridDim.x * blockDim.x) {
@@ -236,7 +247,8 @@ __global__ void __launch_bounds__(256) window_input_kernel(
       if (m != 0.f && seed) v = seed[(long long)b * seed_bs + (long long)f * ch + c];   // no seed yet (first window): motion itself, M.py:379
       m = 0.f;
     }
-    const float o = (m == 1.f) ? mask_embedding[c] : v;   // M.py:267-268
+    float o = (m == 1.f) ? mask_embedding[c] : v;   // M.py:267-268
+    if (win_len_valid && f >= __ldg(win_len_valid + b)) o = 0.f;     // ragged batch: zero rows beyond the clip's window
     if (out) out[i] = o;
     if (P.ptr) pm_store_planes_t<F16>(P, bf, c, o);
   }
@@ -250,11 +262,11 @@ inline int grid_for(long long work, int threads) {
 
 }  // namespace
 
-extern "C" int pm_wav_stem_f32(const float* audio, long long a_bs, long long a_ws, int batch, int windows,
-                               int n_samples, const float* w1, const float* b1, const float* wd,
-                               const float* bd, int cout, int ksize, int stride, int pad, int rows_out,
-                               float slope, float* y1, float* sc,
-                               uint16_t* planes, long long p_ps, int p_ld, int p_nsplit, void* stream) {
+static int wav_stem_run(const float* audio, long long a_bs, long long a_ws, int batch, int windows,
+                        int n_samples, const float* w1, const float* b1, const float* wd,
+                        const float* bd, int cout, int ksize, int stride, int pad, int rows_out,
+                        float slope, float* y1, float* sc,
+                        uint16_t* planes, long long p_ps, int p_ld, int p_nsplit, const int* n_valid, void* stream) {
   PM_REQUIRE(audio && w1 && b1 && wd && bd && sc && (y1 || planes));
   PM_REQUIRE(batch > 0 && windows > 0 && n_samples > 0 && cout > 0 && stride > 0 && rows_out > 0);
   PM_TAKE_FMT(p_nsplit, f16);
@@ -270,11 +282,29 @@ extern "C" int pm_wav_stem_f32(const float* audio, long long a_bs, long long a_w
   cudaStream_t st = (cudaStream_t)stream;
 #define PM_STEM(CO, F)                                                                                          \
   wav_stem_kernel<15, CO, F><<<grid, STEM_THREADS, smem, st>>>(audio, a_bs, a_ws, batch, n_samples, w1, b1, wd, bd, \
-                                                               stride, pad, rows_out, slope, y1, sc, P)
+                                                               stride, pad, rows_out, slope, y1, sc, P, n_valid)
   if (cout == 64) { if (f16) PM_STEM(64, true); else PM_STEM(64, false); }
   else { if (f16) PM_STEM(32, true); else PM_STEM(32, false); }
 #undef PM_STEM
   PM_LAUNCH_CHECK();
+}
+
+extern "C" int pm_wav_stem_f32(const float* audio, long long a_bs, long long a_ws, int batch, int windows,
+                               int n_samples, const float* w1, const float* b1, const float* wd,
+                               const float* bd, int cout, int ksize, int stride, int pad, int rows_out,
+                               float slope, float* y1, float* sc,
+                               uint16_t* planes, long long p_ps, int p_ld, int p_nsplit, void* stream) {
+  return wav_stem_run(audio, a_bs, a_ws, batch, windows, n_samples, w1, b1, wd, bd, cout, ksize, stride, pad, rows_out,
+                      slope, y1, sc, planes, p_ps, p_ld, p_nsplit, nullptr, stream);
+}
+
+extern "C" int pm_wav_stem_rl(const float* audio, long long a_bs, long long a_ws, int batch, int windows,
+                              int n_samples, const float* w1, const float* b1, const float* wd,
+                              const float* bd, int cout, int ksize, int stride, int pad, int rows_out,
+                              float slope, float* y1, float* sc,
+                              uint16_t* planes, long long p_ps, int p_ld, int p_nsplit, const int* n_valid, void* stream) {
+  return wav_stem_run(audio, a_bs, a_ws, batch, windows, n_samples, w1, b1, wd, bd, cout, ksize, stride, pad, rows_out,
+                      slope, y1, sc, planes, p_ps, p_ld, p_nsplit, n_valid, stream);
 }
 
 extern "C" int pm_add_layernorm_f32(const float* x, const float* r, const float* gamma, const float* beta,
@@ -342,10 +372,11 @@ extern "C" int pm_add2_f32(const float* a, const float* b, float* out, long long
   PM_LAUNCH_CHECK();
 }
 
-extern "C" int pm_window_input_f32(const float* motion, const float* mask, const float* seed,
-                                   const float* mask_embedding, float* out, int batch, int total_len,
-                                   int start, int win_len, int pre, int ch, long long seed_bs,
-                                   uint16_t* planes, long long p_ps, int p_ld, int p_nsplit, void* stream) {
+static int window_input_run(const float* motion, const float* mask, const float* seed,
+                            const float* mask_embedding, float* out, int batch, int total_len,
+                            int start, int win_len, int pre, int ch, long long seed_bs,
+                            uint16_t* planes, long long p_ps, int p_ld, int p_nsplit, const int* win_len_valid,
+                            void* stream) {
   PM_REQUIRE(mask_embedding && (out || planes));
   PM_TAKE_FMT(p_nsplit, f16);
   PM_REQUIRE(pm_planes_ok(planes, p_ps, p_ld, p_nsplit, ch, false));
@@ -354,8 +385,25 @@ extern "C" int pm_window_input_f32(const float* motion, const float* mask, const
   const long long total = (long long)batch * win_len * ch;
   if (total == 0) return PM_OK;
   if (f16) window_input_kernel<true><<<grid_for(total, 256), 256, 0, (cudaStream_t)stream>>>(
-      motion, mask, seed, mask_embedding, out, batch, total_len, start, win_len, pre, ch, seed_bs, P);
+      motion, mask, seed, mask_embedding, out, batch, total_len, start, win_len, pre, ch, seed_bs, P, win_len_valid);
   else window_input_kernel<false><<<grid_for(total, 256), 256, 0, (cudaStream_t)stream>>>(
-      motion, mask, seed, mask_embedding, out, batch, total_len, start, win_len, pre, ch, seed_bs, P);
+      motion, mask, seed, mask_embedding, out, batch, total_len, start, win_len, pre, ch, seed_bs, P, win_len_valid);
   PM_LAUNCH_CHECK();
+}
+
+extern "C" int pm_window_input_f32(const float* motion, const float* mask, const float* seed,
+                                   const float* mask_embedding, float* out, int batch, int total_len,
+                                   int start, int win_len, int pre, int ch, long long seed_bs,
+                                   uint16_t* planes, long long p_ps, int p_ld, int p_nsplit, void* stream) {
+  return window_input_run(motion, mask, seed, mask_embedding, out, batch, total_len, start, win_len, pre, ch, seed_bs,
+                          planes, p_ps, p_ld, p_nsplit, nullptr, stream);
+}
+
+extern "C" int pm_window_input_rl(const float* motion, const float* mask, const float* seed,
+                                  const float* mask_embedding, float* out, int batch, int total_len,
+                                  int start, int win_len, int pre, int ch, long long seed_bs,
+                                  uint16_t* planes, long long p_ps, int p_ld, int p_nsplit, const int* win_len_valid,
+                                  void* stream) {
+  return window_input_run(motion, mask, seed, mask_embedding, out, batch, total_len, start, win_len, pre, ch, seed_bs,
+                          planes, p_ps, p_ld, p_nsplit, win_len_valid, stream);
 }

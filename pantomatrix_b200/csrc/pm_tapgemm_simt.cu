@@ -17,6 +17,7 @@ struct TapGemmParams {
   const float* R; long long r_bs; int ldr;
   int act; float slope;
   float* O; long long o_bs; int ldo;
+  const int* row_limit; int rows_per_clip;   // ragged batches (pm_tapgemm_f32_rl), see pm_tapgemm_tc.cu
 };
 
 __global__ void __launch_bounds__(NT) tapgemm_f32_kernel(TapGemmParams p) {
@@ -86,16 +87,51 @@ __global__ void __launch_bounds__(NT) tapgemm_f32_kernel(TapGemmParams p) {
   for (int i = 0; i < 8; ++i) {
     const int l = l0 + ty * 8 + i;
     if (l >= p.rows_out) continue;
+    bool zero = false;                     // beyond its clip's row limit: stored as 0 (negative limit: not stored)
+    if (p.row_limit) {
+      long long clip = b, r = l;
+      if (p.rows_per_clip > 0) {
+        const long long g = (long long)b * p.rows_out + l;
+        clip = g / p.rows_per_clip;
+        r = g - clip * p.rows_per_clip;
+      }
+      const int lim = __ldg(p.row_limit + clip);
+      if (r >= lim) {
+        if (lim < 0) continue;
+        zero = true;
+      }
+    }
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
       const int n = n0 + tx * 4 + j;
       if (n >= p.cout) continue;
+      if (zero) { O[(long long)l * p.ldo + n] = 0.f; continue; }
       float v = acc[i][j];
       if (p.bias) v += __ldg(p.bias + n);
       if (R) v += __ldg(R + (long long)l * p.ldr + n);
       O[(long long)l * p.ldo + n] = pm_act(v, p.act, p.slope);
     }
   }
+}
+
+static int tapgemm_f32_run(const float* A, long long a_bs, int lda, int batch, int rows_in, int cin,
+                           const float* W, const float* bias, int taps, int stride, int pad,
+                           int rows_out, int cout,
+                           const float* residual, long long r_bs, int ldr,
+                           int act, float slope,
+                           float* out, long long o_bs, int ldo, const int* row_limit, int rows_per_clip, void* stream) {
+  PM_REQUIRE(rows_per_clip >= 0);
+  PM_REQUIRE(A && W && out);
+  PM_REQUIRE(batch >= 0 && rows_in >= 0 && rows_out >= 0 && cin > 0 && cout > 0 && taps > 0 && stride > 0);
+  PM_REQUIRE(lda >= cin && ldo >= cout && (!residual || ldr >= cout));
+  PM_REQUIRE(act >= PM_ACT_NONE && act <= PM_ACT_LEAKY);
+  if (batch == 0 || rows_out == 0) return PM_OK;
+  PM_REQUIRE(batch <= 65535);
+  TapGemmParams p{A, a_bs, lda, rows_in, cin, W, bias, taps, stride, pad, rows_out, cout,
+                  residual, r_bs, ldr, act, slope, out, o_bs, ldo, row_limit, rows_per_clip};
+  dim3 grid(pm_cdiv(rows_out, BM), pm_cdiv(cout, BN), batch);
+  tapgemm_f32_kernel<<<grid, NT, 0, (cudaStream_t)stream>>>(p);
+  PM_LAUNCH_CHECK();
 }
 
 }  // namespace
@@ -106,15 +142,17 @@ extern "C" int pm_tapgemm_f32(const float* A, long long a_bs, int lda, int batch
                               const float* residual, long long r_bs, int ldr,
                               int act, float slope,
                               float* out, long long o_bs, int ldo, void* stream) {
-  PM_REQUIRE(A && W && out);
-  PM_REQUIRE(batch >= 0 && rows_in >= 0 && rows_out >= 0 && cin > 0 && cout > 0 && taps > 0 && stride > 0);
-  PM_REQUIRE(lda >= cin && ldo >= cout && (!residual || ldr >= cout));
-  PM_REQUIRE(act >= PM_ACT_NONE && act <= PM_ACT_LEAKY);
-  if (batch == 0 || rows_out == 0) return PM_OK;
-  PM_REQUIRE(batch <= 65535);
-  TapGemmParams p{A, a_bs, lda, rows_in, cin, W, bias, taps, stride, pad, rows_out, cout,
-                  residual, r_bs, ldr, act, slope, out, o_bs, ldo};
-  dim3 grid(pm_cdiv(rows_out, BM), pm_cdiv(cout, BN), batch);
-  tapgemm_f32_kernel<<<grid, NT, 0, (cudaStream_t)stream>>>(p);
-  PM_LAUNCH_CHECK();
+  return tapgemm_f32_run(A, a_bs, lda, batch, rows_in, cin, W, bias, taps, stride, pad, rows_out, cout, residual, r_bs,
+                         ldr, act, slope, out, o_bs, ldo, nullptr, 0, stream);
+}
+
+extern "C" int pm_tapgemm_f32_rl(const float* A, long long a_bs, int lda, int batch, int rows_in, int cin,
+                                 const float* W, const float* bias, int taps, int stride, int pad,
+                                 int rows_out, int cout,
+                                 const float* residual, long long r_bs, int ldr,
+                                 int act, float slope,
+                                 float* out, long long o_bs, int ldo, const int* row_limit, int rows_per_clip,
+                                 void* stream) {
+  return tapgemm_f32_run(A, a_bs, lda, batch, rows_in, cin, W, bias, taps, stride, pad, rows_out, cout, residual, r_bs,
+                         ldr, act, slope, out, o_bs, ldo, row_limit, rows_per_clip, stream);
 }

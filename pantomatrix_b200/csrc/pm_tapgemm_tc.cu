@@ -49,6 +49,9 @@ struct TcParams {
   int stages;
   const uint8_t* prefetch; long long prefetch_bytes;   // next GEMM's weights: pulled into L2 while this one runs
   float acc_scale;   // fp16 operands: weights are packed scaled by a power of two, undone here (1 for bf16)
+  // ragged batches (pm_tapgemm_tc_rl, nullable): row_limit[clip] valid output rows per clip; the clip of output row
+  // (b, l) is b, or (b * rows_out + l) / rows_per_clip when rows_per_clip > 0 (a Linear over all clips as one matrix)
+  const int* row_limit; int rows_per_clip;
 };
 
 // Instrumented build only (-DPM_TC_TIMING, tools/gemm_timeline.py): per-CTA clock64 stamps of the kernel's phases.
@@ -88,7 +91,24 @@ __device__ unsigned long long pm_tc_stamps[4096 * 8];
 // start address that is not 1024-byte aligned needs nothing else - the descriptor's base-offset field must stay 0 (with
 // (start >> 7) & 7 in it, as the PTX text suggests for unaligned starts, every result was wrong).  Only the 8 KB W tiles
 // stream through the ring.  WavEncoder 64 -> 64, k = 15 conv over 0.97 M rows: 444 -> 420 us.
-template <int BN, bool F16, bool CG2, int OCC = 1, bool HALO = false>
+// Ragged batches: 0 = output row (b, l) is computed as usual, 1 = it lies beyond its clip's row limit and is stored as 0,
+// 2 = not stored (outside the output, or a negative limit).  Out of line with scalar arguments: inlined into the
+// two-CTAs-per-SM kernels it raised their register spills; this way they spill less than the plain kernels.
+__device__ __noinline__ int tc_row_limit(const int* __restrict__ row_limit, int rows_per_clip, int batch, int rows_out,
+                                         int b, int l) {
+  if (b >= batch || l >= rows_out) return 2;
+  int clip = b, r = l;
+  if (rows_per_clip > 0) {                                         // batch * rows_out < 2^31 (checked on the host)
+    const int g = b * rows_out + l;
+    clip = g / rows_per_clip;
+    r = g - clip * rows_per_clip;
+  }
+  const int lim = __ldg(row_limit + clip);
+  return r < lim ? 0 : (lim < 0 ? 2 : 1);
+}
+
+// RL = the kernel reads per-clip row limits (pm_tapgemm_tc_rl); without them it compiles to exactly the plain kernel.
+template <int BN, bool F16, bool CG2, int OCC = 1, bool HALO = false, bool RL = false>
 __global__ void __launch_bounds__(NUM_THREADS, OCC) tapgemm_tc_kernel(const __grid_constant__ CUtensorMap map_a,
                                                                     const __grid_constant__ CUtensorMap map_w,
                                                                     const TcParams p) {
@@ -334,6 +354,15 @@ __global__ void __launch_bounds__(NUM_THREADS, OCC) tapgemm_tc_kernel(const __gr
       off_r[i] = (long long)b * p.r_bs + (long long)l * p.ldr;
       off_b[i] = (long long)b * p.ob_bs + (long long)l * p.ldob;
     }
+    // Ragged batch: rows beyond their clip's limit leave the computed set here and are zeroed after the chunk loop,
+    // so the hot loop below is the same code with or without limits (rolled, recomputed: no registers held across it).
+    if (RL && p.row_limit) {
+#pragma unroll 1
+      for (int i = 0; i < NIT; ++i)
+        if (tc_row_limit(p.row_limit, p.rows_per_clip, p.batch, p.rows_out, b0 + ((q * 32 + RPI * i + sub_r) >> r_shift),
+                         l0 + ((q * 32 + RPI * i + sub_r) & (p.R - 1))) != 0)
+          row_ok &= ~(1u << i);
+    }
 #pragma unroll 1
     for (int c0 = half * (BN / 2); c0 < (half + 1) * (BN / 2); c0 += CW) {
       uint32_t acc[CW];
@@ -421,7 +450,7 @@ __global__ void __launch_bounds__(NUM_THREADS, OCC) tapgemm_tc_kernel(const __gr
         for (int i = 0; i < NIT; ++i) {
           const int rt = q * 32 + RPI * i + sub_r;
           const int b = b0 + (rt >> r_shift), l = l0 + (rt & (p.R - 1));
-          if (b >= p.batch || l >= p.rows_out) continue;
+          if (RL ? !((row_ok >> i) & 1u) : (b >= p.batch || l >= p.rows_out)) continue;
           const long long of = (long long)b * p.o_bs + (long long)l * p.ldo;
           const long long orr = (long long)b * p.r_bs + (long long)l * p.ldr;
           const PmPlanes P{p.out_bf16 ? p.out_bf16 + (long long)b * p.ob_bs + (long long)l * p.ldob : nullptr,
@@ -439,6 +468,22 @@ __global__ void __launch_bounds__(NUM_THREADS, OCC) tapgemm_tc_kernel(const __gr
             if (P.ptr) pm_store_planes_t<F16>(P, 0, n + k, y);
           }
         }
+      }
+    }
+  }
+  // Ragged batch: the rows of this CTA beyond their clip's limit, stored as 0 by all 8 epilogue warps (after the
+  // epilogue proper, with nothing it holds in registers: the hot epilogue is the same code with or without limits).
+  if (RL && p.row_limit && warp >= 2) {
+#pragma unroll 1
+    for (int rt = warp - 2; rt < BM; rt += 8) {
+      const int b = blockIdx.z * p.NB + rt / p.R, l = blockIdx.x * p.R + rt % p.R;
+      if (tc_row_limit(p.row_limit, p.rows_per_clip, p.batch, p.rows_out, b, l) != 1) continue;
+      const PmPlanes P{p.out_bf16 ? p.out_bf16 + (long long)b * p.ob_bs + (long long)l * p.ldob : nullptr,
+                       p.ob_ps, p.ldob, p.out_nsplit};
+#pragma unroll 1
+      for (int n = blockIdx.y * BN + lane; n < blockIdx.y * BN + BN && n < p.cout; n += 32) {
+        if (p.out_f32) p.out_f32[(long long)b * p.o_bs + (long long)l * p.ldo + n] = 0.f;
+        if (P.ptr) pm_store_planes_t<F16>(P, 0, n, 0.f);
       }
     }
   }
@@ -486,7 +531,7 @@ __global__ void __launch_bounds__(256) split_bf16_kernel(const float* __restrict
 }
 
 // ---------------------------------------------------------------------------------------------------
-template <int BN, bool F16, bool CG2, int OCC = 1, bool HALO = false>
+template <int BN, bool F16, bool CG2, int OCC = 1, bool HALO = false, bool RL = false>
 int launch(const CUtensorMap& ma, const CUtensorMap& mw, TcParams& p, dim3 grid, cudaStream_t st, int pair_axis = 0) {
   static_assert(OCC == 1 || (BN == 64 && !CG2), "two CTAs per SM: 64-column tiles only (TMEM columns, registers)");
   static_assert(!HALO || (OCC == 2 && BN == 64), "halo mode is built for the 64-column, two-CTAs-per-SM form");
@@ -500,7 +545,7 @@ int launch(const CUtensorMap& ma, const CUtensorMap& mw, TcParams& p, dim3 grid,
   const size_t smem = (size_t)fixed_bytes + (size_t)stages * stage_bytes + 1024 /*align slack*/ + (2 * MAX_STAGES + 3) * sizeof(uint64_t);
   static unsigned long long configured = 0;       // per template instantiation, one bit per device
   if (pm_first_use_on_device(configured)) {
-    cudaError_t e = cudaFuncSetAttribute(tapgemm_tc_kernel<BN, F16, CG2, OCC, HALO>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    cudaError_t e = cudaFuncSetAttribute(tapgemm_tc_kernel<BN, F16, CG2, OCC, HALO, RL>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
     if (e != cudaSuccess) { configured = 0; return (int)e; }
   }
   if constexpr (CG2) {                      // CTA pairs: 2-CTA clusters along the row-tile axis
@@ -516,24 +561,43 @@ int launch(const CUtensorMap& ma, const CUtensorMap& mw, TcParams& p, dim3 grid,
     attr[0].val.clusterDim.z = pair_axis == 2 ? 2 : 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    const cudaError_t e = cudaLaunchKernelEx(&cfg, tapgemm_tc_kernel<BN, F16, CG2, OCC, HALO>, ma, mw, p);
+    const cudaError_t e = cudaLaunchKernelEx(&cfg, tapgemm_tc_kernel<BN, F16, CG2, OCC, HALO, RL>, ma, mw, p);
     return e == cudaSuccess ? PM_OK : (int)e;
   } else {
-    tapgemm_tc_kernel<BN, F16, CG2, OCC, HALO><<<grid, NUM_THREADS, smem, st>>>(ma, mw, p);
+    tapgemm_tc_kernel<BN, F16, CG2, OCC, HALO, RL><<<grid, NUM_THREADS, smem, st>>>(ma, mw, p);
     PM_LAUNCH_CHECK();
   }
 }
 
+template <bool RL>
+int dispatch(const CUtensorMap& ma, const CUtensorMap& mw, TcParams& p, dim3 grid, cudaStream_t st, bool halo, bool f16,
+             bool cg2, bool occ2, int BNsel, int pair_axis) {
+  if (halo) {
+    if (f16) return launch<64, true, false, 2, true, RL>(ma, mw, p, grid, st);
+    return launch<64, false, false, 2, true, RL>(ma, mw, p, grid, st);
+  }
+  if (f16) {
+    if (cg2) return launch<128, true, true, 1, false, RL>(ma, mw, p, grid, st, pair_axis);
+    if (occ2) return launch<64, true, false, 2, false, RL>(ma, mw, p, grid, st);
+    if (BNsel == 64) return launch<64, true, false, 1, false, RL>(ma, mw, p, grid, st);
+    return launch<128, true, false, 1, false, RL>(ma, mw, p, grid, st);
+  }
+  if (occ2) return launch<64, false, false, 2, false, RL>(ma, mw, p, grid, st);
+  if (BNsel == 64) return launch<64, false, false, 1, false, RL>(ma, mw, p, grid, st);
+  return launch<128, false, false, 1, false, RL>(ma, mw, p, grid, st);
+}
+
 }  // namespace
 
-extern "C" int pm_tapgemm_tc(const uint16_t* A, long long a_ps, long long a_bs, int lda, int batch, int rows_in, int cin,
-                             const uint16_t* W, long long w_ps, int w_rows, int ldw, int taps, int pad, int nsplit,
-                             const float* bias, int rows_out, int cout,
-                             const float* residual, long long r_bs, int ldr,
-                             int act, int act_cols, float slope, float acc_scale,
-                             float* out_f32, long long o_bs, int ldo,
-                             uint16_t* out_bf16, long long ob_ps, long long ob_bs, int ldob, int out_nsplit,
-                             const void* prefetch, long long prefetch_bytes, void* stream) {
+static int tapgemm_tc_run(const uint16_t* A, long long a_ps, long long a_bs, int lda, int batch, int rows_in, int cin,
+                          const uint16_t* W, long long w_ps, int w_rows, int ldw, int taps, int pad, int nsplit,
+                          const float* bias, int rows_out, int cout,
+                          const float* residual, long long r_bs, int ldr,
+                          int act, int act_cols, float slope, float acc_scale,
+                          float* out_f32, long long o_bs, int ldo,
+                          uint16_t* out_bf16, long long ob_ps, long long ob_bs, int ldob, int out_nsplit,
+                          const void* prefetch, long long prefetch_bytes, const int* row_limit, int rows_per_clip,
+                          void* stream) {
   PM_REQUIRE(A && W && (out_f32 || out_bf16));
   PM_TAKE_FMT(nsplit, f16);                 // operand planes: bf16 (default) or fp16
   PM_TAKE_FMT(out_nsplit, out_f16);
@@ -588,6 +652,7 @@ extern "C" int pm_tapgemm_tc(const uint16_t* A, long long a_ps, long long a_bs, 
   p.prefetch = static_cast<const uint8_t*>(prefetch);
   p.prefetch_bytes = prefetch ? prefetch_bytes : 0;
   p.acc_scale = acc_scale;
+  p.row_limit = row_limit; p.rows_per_clip = rows_per_clip;
   CUtensorMap ma, mw;
   {
     const long long bs_el = batch > 1 ? a_bs : (long long)rows_in * lda;
@@ -610,19 +675,36 @@ extern "C" int pm_tapgemm_tc(const uint16_t* A, long long a_ps, long long a_bs, 
   static const bool occ2_on = !(getenv("PM_TC_OCC2") && atoi(getenv("PM_TC_OCC2")) == 0);      // A/B switch (tools)
   const bool occ2 = occ2_on && BNsel == 64 && (long long)grid.x * grid.y * grid.z > 2 * 148 &&
                     OCC2_SMEM_KB * 1024 / (nsplit * (A_TILE_BYTES + 64 * BK * 2)) >= 2;
-  if (halo) {
-    if (f16) return launch<64, true, false, 2, true>(ma, mw, p, grid, (cudaStream_t)stream);
-    return launch<64, false, false, 2, true>(ma, mw, p, grid, (cudaStream_t)stream);
-  }
-  if (f16) {
-    if (cg2) return launch<128, true, true>(ma, mw, p, grid, (cudaStream_t)stream, pair_axis);
-    if (occ2) return launch<64, true, false, 2>(ma, mw, p, grid, (cudaStream_t)stream);
-    if (BNsel == 64) return launch<64, true, false>(ma, mw, p, grid, (cudaStream_t)stream);
-    return launch<128, true, false>(ma, mw, p, grid, (cudaStream_t)stream);
-  }
-  if (occ2) return launch<64, false, false, 2>(ma, mw, p, grid, (cudaStream_t)stream);
-  if (BNsel == 64) return launch<64, false, false>(ma, mw, p, grid, (cudaStream_t)stream);
-  return launch<128, false, false>(ma, mw, p, grid, (cudaStream_t)stream);
+  if (row_limit) return dispatch<true>(ma, mw, p, grid, (cudaStream_t)stream, halo, f16, cg2, occ2, BNsel, pair_axis);
+  return dispatch<false>(ma, mw, p, grid, (cudaStream_t)stream, halo, f16, cg2, occ2, BNsel, pair_axis);
+}
+
+extern "C" int pm_tapgemm_tc(const uint16_t* A, long long a_ps, long long a_bs, int lda, int batch, int rows_in, int cin,
+                             const uint16_t* W, long long w_ps, int w_rows, int ldw, int taps, int pad, int nsplit,
+                             const float* bias, int rows_out, int cout,
+                             const float* residual, long long r_bs, int ldr,
+                             int act, int act_cols, float slope, float acc_scale,
+                             float* out_f32, long long o_bs, int ldo,
+                             uint16_t* out_bf16, long long ob_ps, long long ob_bs, int ldob, int out_nsplit,
+                             const void* prefetch, long long prefetch_bytes, void* stream) {
+  return tapgemm_tc_run(A, a_ps, a_bs, lda, batch, rows_in, cin, W, w_ps, w_rows, ldw, taps, pad, nsplit, bias, rows_out,
+                        cout, residual, r_bs, ldr, act, act_cols, slope, acc_scale, out_f32, o_bs, ldo, out_bf16, ob_ps,
+                        ob_bs, ldob, out_nsplit, prefetch, prefetch_bytes, nullptr, 0, stream);
+}
+
+extern "C" int pm_tapgemm_tc_rl(const uint16_t* A, long long a_ps, long long a_bs, int lda, int batch, int rows_in, int cin,
+                                const uint16_t* W, long long w_ps, int w_rows, int ldw, int taps, int pad, int nsplit,
+                                const float* bias, int rows_out, int cout,
+                                const float* residual, long long r_bs, int ldr,
+                                int act, int act_cols, float slope, float acc_scale,
+                                float* out_f32, long long o_bs, int ldo,
+                                uint16_t* out_bf16, long long ob_ps, long long ob_bs, int ldob, int out_nsplit,
+                                const void* prefetch, long long prefetch_bytes, const int* row_limit, int rows_per_clip,
+                                void* stream) {
+  PM_REQUIRE(rows_per_clip >= 0 && (long long)batch * rows_out < (1LL << 31));
+  return tapgemm_tc_run(A, a_ps, a_bs, lda, batch, rows_in, cin, W, w_ps, w_rows, ldw, taps, pad, nsplit, bias, rows_out,
+                        cout, residual, r_bs, ldr, act, act_cols, slope, acc_scale, out_f32, o_bs, ldo, out_bf16, ob_ps,
+                        ob_bs, ldob, out_nsplit, prefetch, prefetch_bytes, row_limit, rows_per_clip, stream);
 }
 
 #ifdef PM_TC_TIMING

@@ -138,7 +138,8 @@ __global__ void __launch_bounds__(256) row_argmax_kernel(const float* __restrict
 template <bool F16>
 __global__ void __launch_bounds__(256) gather_rows_kernel(const float* __restrict__ codebook, long long n_table,
                                                           const long long* __restrict__ index, long long rows,
-                                                          int ch4, float* __restrict__ out, PmPlanes P) {
+                                                          int ch4, float* __restrict__ out, PmPlanes P,
+                                                          const int* __restrict__ row_limit, int rows_per_clip) {
   const long long total = rows * ch4;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total;
        i += (long long)gridDim.x * blockDim.x) {
@@ -146,7 +147,8 @@ __global__ void __launch_bounds__(256) gather_rows_kernel(const float* __restric
     const int c4 = (int)(i % ch4);
     long long k = index[r];                       // out-of-range ids (user input) are clamped: never read outside the table
     k = k < 0 ? 0 : (k >= n_table ? n_table - 1 : k);
-    const float4 v = reinterpret_cast<const float4*>(codebook)[k * ch4 + c4];
+    float4 v = reinterpret_cast<const float4*>(codebook)[k * ch4 + c4];
+    if (row_limit && r % rows_per_clip >= __ldg(row_limit + r / rows_per_clip)) v = make_float4(0.f, 0.f, 0.f, 0.f);
     if (out) reinterpret_cast<float4*>(out)[i] = v;
     if (P.ptr) pm_store_planes4_t<F16>(P, r, c4 * 4, v);
   }
@@ -205,19 +207,35 @@ extern "C" int pm_row_argmax_f32(const float* x, long long rows, int ch, int ldx
   PM_LAUNCH_CHECK();
 }
 
-extern "C" int pm_gather_rows_f32(const float* codebook, long long n_table, const long long* index, long long rows, int ch,
-                                  float* out, uint16_t* planes, long long p_ps, int p_ld, int p_nsplit,
-                                  void* stream) {
+static int gather_rows_run(const float* codebook, long long n_table, const long long* index, long long rows, int ch,
+                           float* out, uint16_t* planes, long long p_ps, int p_ld, int p_nsplit,
+                           const int* row_limit, int rows_per_clip, void* stream) {
   PM_REQUIRE(codebook && index && (out || planes) && rows >= 0 && n_table > 0 && ch > 0 && (ch & 3) == 0);
+  PM_REQUIRE(!row_limit || rows_per_clip > 0);
   PM_TAKE_FMT(p_nsplit, f16);
   PM_REQUIRE(pm_planes_ok(planes, p_ps, p_ld, p_nsplit, ch, true));
   const PmPlanes P{reinterpret_cast<__nv_bfloat16*>(planes), p_ps, p_ld, p_nsplit};
   if (rows == 0) return PM_OK;
   long long g = (rows * (ch >> 2) + 255) / 256;
   if (g > 148 * 16) g = 148 * 16;
-  if (f16) gather_rows_kernel<true><<<(unsigned)g, 256, 0, (cudaStream_t)stream>>>(codebook, n_table, index, rows, ch >> 2, out, P);
-  else gather_rows_kernel<false><<<(unsigned)g, 256, 0, (cudaStream_t)stream>>>(codebook, n_table, index, rows, ch >> 2, out, P);
+  if (f16) gather_rows_kernel<true><<<(unsigned)g, 256, 0, (cudaStream_t)stream>>>(codebook, n_table, index, rows, ch >> 2, out, P,
+                                                                                   row_limit, rows_per_clip);
+  else gather_rows_kernel<false><<<(unsigned)g, 256, 0, (cudaStream_t)stream>>>(codebook, n_table, index, rows, ch >> 2, out, P,
+                                                                                 row_limit, rows_per_clip);
   PM_LAUNCH_CHECK();
+}
+
+extern "C" int pm_gather_rows_f32(const float* codebook, long long n_table, const long long* index, long long rows, int ch,
+                                  float* out, uint16_t* planes, long long p_ps, int p_ld, int p_nsplit,
+                                  void* stream) {
+  return gather_rows_run(codebook, n_table, index, rows, ch, out, planes, p_ps, p_ld, p_nsplit, nullptr, 0, stream);
+}
+
+extern "C" int pm_gather_rows_rl(const float* codebook, long long n_table, const long long* index, long long rows, int ch,
+                                 float* out, uint16_t* planes, long long p_ps, int p_ld, int p_nsplit,
+                                 const int* row_limit, int rows_per_clip, void* stream) {
+  return gather_rows_run(codebook, n_table, index, rows, ch, out, planes, p_ps, p_ld, p_nsplit, row_limit, rows_per_clip,
+                         stream);
 }
 
 extern "C" int pm_row_sqnorm_f32(const float* x, int rows, int ch, float* out, void* stream) {

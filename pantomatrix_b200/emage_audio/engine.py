@@ -18,9 +18,10 @@ Schedule differences from the reference that do not change results beyond fp32 r
 """
 from __future__ import annotations
 
+import numpy as np
 import torch
 
-from .. import ops
+from .. import _lib, ops
 
 PARTS = ("face", "upper", "hands", "lower")
 # WavEncoder geometry P.py:300-307: (stride, first-conv padding, has downsample branch)
@@ -39,12 +40,19 @@ def _fold_bn(sd, conv, bn, eps=1e-5):
     return (w * s[:, None, None]).float(), ((b - sd[bn + ".running_mean"].double()) * s + sd[bn + ".bias"].double()).float()
 
 
-def wav_out_len(n: int) -> int:
-    """Frames a WavEncoder emits for n samples (P.py:300-307 conv arithmetic)."""
-    length = n
+def wav_block_lens(n: int) -> list[int]:
+    """Rows each WavEncoder block emits for n samples (P.py:300-307 conv arithmetic); a block's k=15 / pad 7 second
+    conv keeps the row count of its first."""
+    lens, length = [], n
     for stride, pad, _ in WAV_BLOCKS:
         length = (length + 2 * pad - 15) // stride + 1
-    return length
+        lens.append(length)
+    return lens
+
+
+def wav_out_len(n: int) -> int:
+    """Frames a WavEncoder emits for n samples (P.py:300-307 conv arithmetic)."""
+    return wav_block_lens(n)[-1]
 
 
 # Arithmetic engine of every Conv1d / Linear ("tap-GEMM"): 0 = fp32 SIMT kernel, 1/2/3 = tcgen05 tensor cores with
@@ -194,15 +202,17 @@ class _Conv:
             self._packed[key] = ops.PackedW(w, nsplit)
         return self._packed[key]
 
-    def __call__(self, x, act=ops.ACT_NONE, slope=0.0, residual=None, out=None, want="f", out_slack=0):
+    def __call__(self, x, act=ops.ACT_NONE, slope=0.0, residual=None, out=None, want="f", out_slack=0, row_limit=None):
         """x: fp32 tensor, ops.Planes or ops.Act.  want: "f" (fp32 tensor returned), "p" (bf16 planes only) or
         "fp" (both); with planes requested an ops.Act is returned.  In fp32 mode planes do not exist: the fp32
-        tensor is always produced and returned (wrapped in an Act when planes were asked for)."""
+        tensor is always produced and returned (wrapped in an Act when planes were asked for).
+        row_limit: per-clip valid output rows of a ragged batch (int32 device tensor, None = all rows)."""
         ns = _STATE["nsplit"]
         residual = _f32(residual)
+        lim = {} if row_limit is None else {"row_limit": row_limit}          # no limit: exactly the plain call
         if ns == 0:
             y = ops.tapgemm(_f32(x), self.w, self.b, stride=self.stride, pad=self.pad, act=act, slope=slope,
-                            residual=residual, out=out)
+                            residual=residual, out=out, **lim)
             return y if want == "f" else ops.Act(y, None)
         taps, cout, _ = self.w.shape
         s = self.stride
@@ -220,13 +230,14 @@ class _Conv:
                 _, pl = ops.tapgemm_tc(a.flat(), self.packed(ns), self.b, rows_out=batch * rows, act=act, slope=slope,
                                        want_f32=want_f, out=None if out is None else out.view(1, batch * rows, cout),
                                        residual=None if residual is None else residual.view(1, batch * rows, cout),
-                                       out_nsplit=out_ns, out_slack=out_slack, prefetch=pf)
+                                       out_nsplit=out_ns, out_slack=out_slack, prefetch=pf,
+                                       **({} if row_limit is None else {"row_limit": row_limit, "rows_per_clip": rows}))
                 if pl is not None:                         # back to the (clips, rows) view
                     pl = ops.Planes(pl.t.view(pl.t.shape[0], batch, rows, pl.t.shape[3]), rows, cout, pl.slack)
             else:
                 _, pl = ops.tapgemm_tc(a, self.packed(ns), self.b, rows_out=rows_out, pad=self.pad, act=act, slope=slope,
                                        residual=residual, want_f32=want_f, out=out, out_nsplit=out_ns, out_slack=out_slack,
-                                       prefetch=pf)
+                                       prefetch=pf, **lim)
             return out if want == "f" else ops.Act(out, pl)
         assert self.pad == 0
         a = _planes(x, ns, need_slack=s)
@@ -235,7 +246,7 @@ class _Conv:
         rows_out = (rows - taps) // s + 1
         o, pl = ops.tapgemm_tc(a, self.packed(ns), self.b, rows_out=rows_out, act=act, slope=slope, residual=residual,
                                want_f32=want_f, out=out, out_nsplit=out_ns, out_slack=out_slack, prefetch=pf,
-                               a_view=(-(-rows // s), s * cin, s * cin))
+                               a_view=(-(-rows // s), s * cin, s * cin), **lim)
         return o if want == "f" else ops.Act(o, pl)
 
 
@@ -276,8 +287,9 @@ class _MLP:
     def __init__(self, sd, p):
         self.fc1, self.fc2 = _Linear(sd, p + ".fc1"), _Linear(sd, p + ".fc2")
 
-    def __call__(self, x, out=None, want="f"):
-        return self.fc2(self.fc1(x, act=ops.ACT_LEAKY, slope=0.1, want="p"), out=out, want=want)
+    def __call__(self, x, out=None, want="f", row_limit=None):
+        return self.fc2(self.fc1(x, act=ops.ACT_LEAKY, slope=0.1, want="p", row_limit=row_limit), out=out, want=want,
+                        row_limit=row_limit)
 
 
 class _ConvStack:
@@ -297,16 +309,18 @@ class _ConvStack:
                 self.steps.append(("conv", c(2 + 2 * i), True))
             self.steps.append(("conv", c(2 + 2 * n_layer), False))
 
-    def __call__(self, x, want="f"):
+    def __call__(self, x, want="f", row_limit=None):
         """x: tensor / Act (a ResBlock needs its fp32 copy for the skip).  Intermediate activations travel as
-        fp32 + bf16 planes; only the last step honours `want`."""
+        fp32 + bf16 planes; only the last step honours `want`.  row_limit: per-clip valid rows of a ragged batch -
+        every conv zeroes the rows beyond, which is the zero padding the next conv of the clip alone would read."""
         last = len(self.steps) - 1
+        rl = row_limit
         for i, step in enumerate(self.steps):
             w = want if i == last else "fp"
             if step[0] == "conv":
-                x = step[1](x, act=ops.ACT_LEAKY if step[2] else ops.ACT_NONE, slope=0.2, want=w)
+                x = step[1](x, act=ops.ACT_LEAKY if step[2] else ops.ACT_NONE, slope=0.2, want=w, row_limit=rl)
             else:
-                x = step[2](step[1](x, act=ops.ACT_LEAKY, slope=0.2, want="p"), residual=x, want=w)
+                x = step[2](step[1](x, act=ops.ACT_LEAKY, slope=0.2, want="p", row_limit=rl), residual=x, want=w, row_limit=rl)
         return x
 
 
@@ -328,22 +342,25 @@ class _WavEncoder:
                 self.blocks.append((_Conv(_taps(w1), b1.contiguous(), stride, pad), _Conv(_taps(w2), b2.contiguous(), 1, 7),
                                     _Conv(_taps(ds[0]), ds[1].contiguous(), stride, pad) if ds else None))
 
-    def __call__(self, audio, offset, a_ws, windows, n_samples):
-        """audio (bs, n) contiguous; returns (windows*bs, frames, out_dim), window-major."""
+    def __call__(self, audio, offset, a_ws, windows, n_samples, limits=None):
+        """audio (bs, n) contiguous; returns (windows*bs, frames, out_dim), window-major.
+        limits: ragged batch - (samples per slice, [valid rows after each block]), int32 device tensors over the
+        window-major slices (RaggedPlan); None: every slice is n_samples long."""
         bs, n = audio.shape
         w1, b1, wd, bd, stride, pad = self.stem
+        n_valid, rows = limits if limits is not None else (None, [None] * len(self.blocks))
         y, sc = ops.wav_stem(audio, n, a_ws, bs, windows, n_samples, w1, b1, wd, bd, stride=stride, pad=pad,
-                             slope=0.01, offset=offset, nsplit=_ns())
+                             slope=0.01, offset=offset, nsplit=_ns(), **({} if n_valid is None else {"n_valid": n_valid}))
         # A block's output feeds the next block's convs as (possibly strided) GEMM operand - planes - and, only where
         # that block has no downsample conv, as its identity shortcut - fp32.  (The first block's output is 0.25 GB
         # per encoder in fp32 at the BASELINE batch: not writing it is the point.)
         last = len(self.blocks) - 1
         form = lambda i: "f" if i == last else ("p" if self.blocks[i + 1][2] is not None else "fp")
-        x = self.blocks[0][1](y, act=ops.ACT_LEAKY, slope=0.01, residual=sc, want=form(0), out_slack=8)
+        x = self.blocks[0][1](y, act=ops.ACT_LEAKY, slope=0.01, residual=sc, want=form(0), out_slack=8, row_limit=rows[0])
         for i, (conv1, conv2, ds) in enumerate(self.blocks[1:], 1):
-            y = conv1(x, act=ops.ACT_LEAKY, slope=0.01, want="p")
-            sc = ds(x) if ds is not None else x
-            x = conv2(y, act=ops.ACT_LEAKY, slope=0.01, residual=sc, want=form(i), out_slack=8)
+            y = conv1(x, act=ops.ACT_LEAKY, slope=0.01, want="p", row_limit=rows[i])
+            sc = ds(x) if ds is not None else x          # only read as conv2's residual, on rows conv2 computes
+            x = conv2(y, act=ops.ACT_LEAKY, slope=0.01, residual=sc, want=form(i), out_slack=8, row_limit=rows[i])
         return x
 
 
@@ -375,8 +392,11 @@ class _Layer:
         the tensor-core attention kernel reads in place."""
         return self.ca.kv(mem, want="p" if _attn_tc() else "f")
 
-    def __call__(self, x, mem_kv=None, want="f"):
-        """x: fp32 tensor or Act(f, p) of (bs, t, E).  Returns the layer output in the requested form."""
+    def __call__(self, x, mem_kv=None, want="f", q_len=None, k_len=None):
+        """x: fp32 tensor or Act(f, p) of (bs, t, E).  Returns the layer output in the requested form.
+        Ragged batch: q_len = per-clip valid rows of x (the self-attention keys too), k_len = per-clip memory keys."""
+        sa = {} if q_len is None else {"q_len": q_len, "k_len": q_len}
+        ca = {} if q_len is None else {"q_len": q_len, "k_len": k_len}
         ns = _ns()
         xf = _f32(x)
         bs, t, E = xf.shape
@@ -384,22 +404,22 @@ class _Layer:
         tc = _attn_tc()
         if tc:                                  # packed q|k|v planes straight from the GEMM epilogue, read in place by TMA
             qkv = self.sa.qkv(x, want="p").p
-            att = ops.attention_tc(qkv, 0, qkv, E, qkv, 2 * E, bs, NHEAD, t, t, hd, nsplit=ns)
+            att = ops.attention_tc(qkv, 0, qkv, E, qkv, 2 * E, bs, NHEAD, t, t, hd, nsplit=ns, **sa)
         else:
             qkv = self.sa.qkv(x).view(bs * t, 3 * E)
-            att = ops.attention(qkv[:, :E], qkv[:, E:2 * E], qkv[:, 2 * E:], bs, NHEAD, t, t, hd, nsplit=ns, f32=ns == 0)
+            att = ops.attention(qkv[:, :E], qkv[:, E:2 * E], qkv[:, 2 * E:], bs, NHEAD, t, t, hd, nsplit=ns, f32=ns == 0, **sa)
         x = ops.add_layernorm(self.sa.out(_view3(att, bs, t, E), residual=xf), None, *self.norms[0], nsplit=ns)
         k = 1
         if self.ca is not None:
             if tc:
                 kv = mem_kv.p if isinstance(mem_kv, ops.Act) else mem_kv
-                att = ops.attention_tc(self.ca.q(x, want="p").p, 0, kv, 0, kv, E, bs, NHEAD, t, kv.rows, hd, nsplit=ns)
+                att = ops.attention_tc(self.ca.q(x, want="p").p, 0, kv, 0, kv, E, bs, NHEAD, t, kv.rows, hd, nsplit=ns, **ca)
             else:
                 tk = mem_kv.shape[1]
                 assert mem_kv.is_contiguous()
                 kv = mem_kv.view(bs * tk, 2 * E)
                 q = self.ca.q(x).view(bs * t, E)
-                att = ops.attention(q, kv[:, :E], kv[:, E:], bs, NHEAD, t, tk, hd, nsplit=ns, f32=ns == 0)
+                att = ops.attention(q, kv[:, :E], kv[:, E:], bs, NHEAD, t, tk, hd, nsplit=ns, f32=ns == 0, **ca)
             x = ops.add_layernorm(self.ca.out(_view3(att, bs, t, E), residual=_f32(x)), None, *self.norms[1], nsplit=ns)
             k = 2
         h = self.l1(x, act=ops.ACT_RELU, want="p")
@@ -462,19 +482,20 @@ class EmageEngine:
         self._lane_forks = {}          # clip-group lane -> (face || body fork, refine-parts fork): side streams are per lane
 
     # ------------------------------------------------------------------------------------------------
-    def audio_phase(self, audio, offset, a_ws, windows, n_samples, t):
+    def audio_phase(self, audio, offset, a_ws, windows, n_samples, t, limits=None):
         """Everything that depends on audio only, for `windows` equally long slices per clip.
         Returns window-major tensors: face memory audio part (w*bs, t, E), body cross-attn K|V of the
-        8 layers (list of (w*bs, tk, 2E))."""
+        8 layers (list of (w*bs, tk, 2E)).  limits: a ragged batch's WavEncoder limits (RaggedLimits.wav)."""
         if wav_out_len(n_samples) < t:
             raise ValueError(f"audio slice yields {wav_out_len(n_samples)} frames < {t} motion frames")
+        wl = {} if limits is None else {"limits": limits}
 
         def face():
-            a_face = self.wav_face(audio, offset, a_ws, windows, n_samples)
+            a_face = self.wav_face(audio, offset, a_ws, windows, n_samples, **wl)
             return self.face_mem_audio(a_face[:, :t])      # M.py:278-281 (the body stream is never truncated)
 
         def body():
-            mem_body = self.body_mem(self.wav_body(audio, offset, a_ws, windows, n_samples), want="p" if _ns() else "f")
+            mem_body = self.body_mem(self.wav_body(audio, offset, a_ws, windows, n_samples, **wl), want="p" if _ns() else "f")
             return [layer.project_memory(mem_body) for layer in self.cross]
 
         kv, mem_face = self._fork_audio.run([body, face])
@@ -485,12 +506,19 @@ class EmageEngine:
             self._lane_forks[lane] = (_Fork(1), _Fork(2))
         return self._lane_forks[lane]
 
-    def window(self, win_in, speaker_id_rows, mem_face_audio, kv_body, dest=None, use_audio=True, lane=0):
+    def window(self, win_in, speaker_id_rows, mem_face_audio, kv_body, dest=None, use_audio=True, lane=0, limits=None):
         """One window of EmageAudioModel.forward (M.py:265-341) given the hoisted audio tensors.
         win_in (bs,t,337) is already mask-embedded.  speaker_id_rows = (spk_face_rows, spk_body_rows).
         dest: optional dict name -> (bs, t, 256) fp32 view the final GEMM of that output writes into (the window's rows
-        of inference()'s accumulated outputs), so nothing is copied afterwards."""
+        of inference()'s accumulated outputs), so nothing is copied afterwards.
+        limits: ragged batch - per-clip (rows, body memory keys, rows written to dest) of this window, int32 device
+        tensors (RaggedLimits.window); None: every clip has t rows."""
         dest = dest or {}
+        rows, tk, dest_rows = limits if limits is not None else (None, None, None)
+        rl = {} if rows is None else {"row_limit": rows}
+        self_kq = {} if rows is None else {"q_len": rows, "k_len": rows}
+        cross_k = {} if rows is None else {"q_len": rows, "k_len": tk}
+        out_rl = {} if rows is None else {"row_limit": dest_rows}
         fork_branch, fork_parts = self._forks(lane)
         # use_audio=False (training-time ablation, M.py:310-311): the body's audio cross-attention output is multiplied
         # by zero, i.e. motion_fea + 0 - the 8 cross layers are simply not run; the face branch still sees the audio.
@@ -498,26 +526,26 @@ class EmageEngine:
         E = self.E
         spk_f, spk_b = speaker_id_rows
         ns = _ns()
-        hint = self.motion_encoder(win_in, want="p" if ns else "f")                    # M.py:271
+        hint = self.motion_encoder(win_in, want="p" if ns else "f", **rl)              # M.py:271
 
         def face_branch():                                                              # M.py:288-294
             hint_face = self.hint_face(hint, want="p" if ns else "f")
             mem_f = self.face_mem_hint(hint_face, residual=mem_face_audio, want="p" if ns else "f")
             x = ops.add_rows(None, self.pe, spk_f, ops.ROW_SPK, ops.ROW_PE, bs, t, E, nsplit=ns)
             for i, layer in enumerate(self.face_dec):
-                x = layer(x, layer.project_memory(mem_f), want="fp" if i + 1 < len(self.face_dec) else "p")
-            rec = self.out_proj["face"](x, want="fp", out=dest.get("rec_face"))
-            return {"rec_face": _f32(rec), "cls_face": self.cls["face"](rec, out=dest.get("cls_face"))}
+                x = layer(x, layer.project_memory(mem_f), want="fp" if i + 1 < len(self.face_dec) else "p", **self_kq)
+            rec = self.out_proj["face"](x, want="fp", out=dest.get("rec_face"), **out_rl)
+            return {"rec_face": _f32(rec), "cls_face": self.cls["face"](rec, out=dest.get("cls_face"), **out_rl)}
 
         def body_branch():                                                              # M.py:297-330
             hint_body = self.hint_body(hint, want="p" if ns else "f")
             x = ops.add_rows(self.moton_proj(hint_body), self.pe, spk_b, ops.ROW_PE, ops.ROW_SPK, bs, t, E, nsplit=ns)
-            fea = self.self_enc(x)
+            fea = self.self_enc(x, **self_kq)
             fea = ops.add_rows(fea, self.pe, spk_b, ops.ROW_SPK, ops.ROW_PE, bs, t, E, nsplit=ns)
             x = fea
             if use_audio:
                 for i, (layer, kv) in enumerate(zip(self.cross, kv_body)):
-                    x = layer(x, kv, want="fp" if i + 1 < len(self.cross) else "f")
+                    x = layer(x, kv, want="fp" if i + 1 < len(self.cross) else "f", **cross_k)
                 fea = ops.add2(_f32(fea), _f32(x), nsplit=ns, f32=ns == 0)
             else:
                 fea = ops.add2(_f32(fea), torch.zeros_like(_f32(fea)), nsplit=ns, f32=ns == 0)
@@ -529,9 +557,10 @@ class EmageEngine:
                 layer = self.refine[p]
                 tgt = ops.add_rows(lat[p], self.pe, spk_b, ops.ROW_SPK, ops.ROW_NONE, bs, t, E, nsplit=ns)
                 mem = ops.add2(lat[a], lat[b], nsplit=ns, f32=ns == 0)
-                r = layer(tgt, layer.project_memory(mem))
-                rec = self.out_proj[p](ops.add2(lat[p], r, nsplit=ns, f32=ns == 0), want="fp", out=dest.get("rec_" + p))
-                return {"rec_" + p: _f32(rec), "cls_" + p: self.cls[p](rec, out=dest.get("cls_" + p))}
+                r = layer(tgt, layer.project_memory(mem), **self_kq)
+                rec = self.out_proj[p](ops.add2(lat[p], r, nsplit=ns, f32=ns == 0), want="fp", out=dest.get("rec_" + p),
+                                       **out_rl)
+                return {"rec_" + p: _f32(rec), "cls_" + p: self.cls[p](rec, out=dest.get("cls_" + p), **out_rl)}
 
             out = {}
             for d in fork_parts.run([lambda p=p: refine(p) for p in PARTS[1:]]):
@@ -571,20 +600,26 @@ class VQEngine:
         self.device = self.codebook["face"].device
         self._forks = {}               # clip-group lane -> fork of the four part decoders
 
-    def part_decode(self, p, index=None, latent=None):
-        """EmageVQVAEConv.decode / decode_from_latent (M.py:56-70) -> (pose features, indices)."""
+    def part_decode(self, p, index=None, latent=None, row_limit=None):
+        """EmageVQVAEConv.decode / decode_from_latent (M.py:56-70) -> (pose features, indices).
+        row_limit: per-clip frame counts of a ragged batch (int32 device tensor), None = all rows."""
         if index is None:                           # latent: (bs, t, 256), dense rows, any clip stride (a window's tail)
             index = ops.l2_argmin(latent, self.codebook[p], self.e2[p])
-        return self.decoder[p](ops.gather_rows(self.codebook[p], index.contiguous(), nsplit=_ns())), index
+        if row_limit is None:
+            return self.decoder[p](ops.gather_rows(self.codebook[p], index.contiguous(), nsplit=_ns())), index
+        x = ops.gather_rows(self.codebook[p], index.contiguous(), nsplit=_ns(), row_limit=row_limit)
+        return self.decoder[p](x, row_limit=row_limit), index
 
-    def decode(self, index, latent, get_global_motion=False, ref_trans=None, lane=0):
-        """index/latent: dicts part -> tensor or None.  Returns the reference's 4-key dict (M.py:193)."""
+    def decode(self, index, latent, get_global_motion=False, ref_trans=None, lane=0, row_limit=None):
+        """index/latent: dicts part -> tensor or None.  Returns the reference's 4-key dict (M.py:193).
+        row_limit: per-clip frame counts of a ragged batch: every conv zeroes the frames beyond."""
         shape = next(t.shape[:2] for t in list(index.values()) + list(latent.values()) if t is not None)
         bs, t = int(shape[0]), int(shape[1])
         todo = [p for p in PARTS if index.get(p) is not None or latent.get(p) is not None]
         if lane not in self._forks:
             self._forks[lane] = _Fork(3)
-        done = self._forks[lane].run([lambda p=p: self.part_decode(p, index.get(p), latent.get(p))[0] for p in todo])
+        done = self._forks[lane].run([lambda p=p: self.part_decode(p, index.get(p), latent.get(p), row_limit=row_limit)[0]
+                                      for p in todo])
         feats = dict(zip(todo, done))
         expression, aa, m4 = ops.pose_compose(feats.get("face"), feats.get("upper"), feats.get("hands"),
                                               feats.get("lower"), bs, t, self.device)
@@ -595,12 +630,13 @@ class VQEngine:
                 lower_mix = torch.zeros(bs, t, 61, device=self.device)
                 lower_mix[:, :, 0:54:6] = 1.0
                 lower_mix[:, :, 4:54:6] = 1.0
-            trans = self.global_motion(lower_mix, ref_trans)
+            trans = self.global_motion(lower_mix, ref_trans, row_limit=row_limit)
         return dict(expression=expression, all_motion4inference=m4, motion_axis_angle=aa, trans=trans)
 
-    def global_motion(self, lower_mix, ref_trans):
+    def global_motion(self, lower_mix, ref_trans, row_limit=None):
         """M.py:195-205."""
-        rec = self.global_dec(self.global_enc(lower_mix))
+        rl = {} if row_limit is None else {"row_limit": row_limit}
+        rec = self.global_dec(self.global_enc(lower_mix, **rl), **rl)
         bs = rec.shape[0]
         ref_trans = ref_trans.to(device=rec.device, dtype=torch.float32)
         if ref_trans.dim() == 2:                    # (n,3) -> every clip starts at row 0 (M.py:198-201)
@@ -735,4 +771,168 @@ def run_inference(engine: EmageEngine, vq: VQEngine, audio, speaker_id, masked_m
         engine._fork_lanes.run([lambda lane=lane: run_lane(lane) for lane in range(n_groups)])
     if pad:
         acc = {k: v[:, :out_len].contiguous() for k, v in acc.items()}
+    return acc
+
+
+# ------------------------------------------------------------------------------------------------------
+# Ragged batches: clips of different lengths in one batched schedule
+# ------------------------------------------------------------------------------------------------------
+
+
+class RaggedPlan:
+    """Per-clip geometry of a ragged batch (host only).  Every clip is laid out at one capacity - `windows` windows of
+    `window` rows for each of `batch` clips - and the int32 tables below say which rows of each (window, clip) are real.
+    Window j of every clip starts at frame j*step and audio sample j*step*spf, as in run_inference().
+
+      win_rows (W, B)      rows of clip b's window j: `window` for a full window, pre + remain for its tail window,
+                           0 where the clip has no window j (window_plan, M.py:365-368)
+      n_valid  (W, B)      audio samples of that window's slice: win_rows * spf
+      wav_rows (6, W, B)   valid rows after each WavEncoder block (wav_block_lens of n_valid; 0 for empty slices)
+      body_keys (W, B)     body cross-attention keys = wav_out_len(n_valid): the body stream is never truncated
+                           (M.py:278-281), so a tail of T <= 25 rows has T + 1 keys
+      dest_rows (W, B)     rows the window writes into the accumulated outputs: win_rows, -1 (nothing) where empty
+      out_len  (B,)        emitted frames per clip
+    """
+
+    def __init__(self, n_samples, window, pre, batch=None, windows=None):
+        n_samples = [int(n) for n in n_samples]
+        self.window, self.pre, self.step, self.spf = window, pre, window - pre, 16000 // 30
+        plans = [window_plan(n * 30 // 16000, window, pre) for n in n_samples]                  # M.py:345
+        if any(not p or p[0][0] < 0 for p in plans):              # (fewer frames than `pre`: a window before frame 0)
+            raise RuntimeError("audio too short: no window to generate (reference torch.cat of an empty list fails too)")
+        self.batch = len(n_samples) if batch is None else int(batch)
+        self.windows = max(len(p) for p in plans) if windows is None else int(windows)
+        if len(n_samples) > self.batch or max(len(p) for p in plans) > self.windows:
+            raise ValueError(f"{len(n_samples)} clips / {max(len(p) for p in plans)} windows exceed the capacity "
+                             f"of {self.batch} clips x {self.windows} windows")
+        W, B = self.windows, self.batch
+        self.win_rows = np.zeros((W, B), np.int32)
+        self.out_len = np.zeros(B, np.int32)
+        for b, plan in enumerate(plans):
+            for j, (s, e, _) in enumerate(plan):
+                assert s == j * self.step
+                self.win_rows[j, b] = e - s
+            self.out_len[b] = sum(k for _, _, k in plan)
+        self.n_valid = self.win_rows * self.spf
+        self.wav_rows = np.zeros((len(WAV_BLOCKS), W, B), np.int32)
+        for j in range(W):
+            for b in range(B):
+                if self.win_rows[j, b]:
+                    self.wav_rows[:, j, b] = wav_block_lens(int(self.n_valid[j, b]))
+        self.body_keys = self.wav_rows[-1].copy()
+        self.dest_rows = np.where(self.win_rows > 0, self.win_rows, -1).astype(np.int32)
+        self.n_clips = len(n_samples)
+
+    @property
+    def capacity_frames(self):
+        return self.windows * self.step + self.pre
+
+    @property
+    def capacity_samples(self):
+        """Audio samples the windows read: a clip's samples beyond this (the fraction of a frame after its last frame,
+        or the frames of a dropped tail, M.py:380-382) are never part of any window."""
+        return ((self.windows - 1) * self.step + self.window) * self.spf
+
+    def tables(self):
+        """name -> int32 array, in the layout RaggedLimits keeps on the device (slices window-major)."""
+        W, B = self.windows, self.batch
+        return {"n_valid": self.n_valid.reshape(W * B), "wav_rows": self.wav_rows.reshape(-1, W * B),
+                "win_rows": self.win_rows, "body_keys": self.body_keys, "dest_rows": self.dest_rows,
+                "out_len": self.out_len}
+
+
+class RaggedLimits:
+    """The tables of a RaggedPlan as int32 device tensors, the per-clip limit arguments of the `_rl` kernels.  All tables
+    are views of one device buffer, so a plan loads with one host -> device copy; they keep their addresses across
+    load() calls, so a graph captured with them reads whatever was loaded last."""
+
+    def __init__(self, plan: RaggedPlan, device):
+        tables = plan.tables()
+        self.buf = torch.empty(sum(v.size for v in tables.values()), dtype=torch.int32, device=device)
+        self.t, off = {}, 0
+        for k, v in tables.items():
+            self.t[k] = self.buf[off:off + v.size].view(v.shape)
+            off += v.size
+        self.windows, self.batch = plan.windows, plan.batch
+        self.load(plan)
+
+    def load(self, plan: RaggedPlan):
+        assert (plan.windows, plan.batch) == (self.windows, self.batch)
+        host = np.concatenate([v.ravel() for v in plan.tables().values()]).astype(np.int32)
+        self.buf.copy_(torch.from_numpy(host))
+
+    @property
+    def wav(self):
+        return self.t["n_valid"], list(self.t["wav_rows"])
+
+    def window(self, j, g0, g1):
+        return self.t["win_rows"][j, g0:g1], self.t["body_keys"][j, g0:g1], self.t["dest_rows"][j, g0:g1]
+
+    @property
+    def out_len(self):
+        return self.t["out_len"]
+
+
+def run_inference_ragged(engine: EmageEngine, vq: VQEngine, audio_padded, limits: RaggedLimits, speaker_id):
+    """run_inference() for a ragged batch laid out at capacity: audio_padded (B, >= capacity samples), zero beyond
+    each clip; limits = the batch's RaggedLimits.  Returns the accumulated rec_* / cls_* outputs (B, capacity frames,
+    256): clip b's outputs are its first out_len[b] rows, equal to run_inference() of that clip alone."""
+    cfg = engine.cfg
+    dev = engine.device
+    window, pre = int(cfg["pose_length"]), int(cfg["seed_frames"])
+    step, spf = window - pre, 16000 // 30
+    ch = int(cfg["pose_dims"]) + 7
+    W, B = limits.windows, limits.batch
+    audio = audio_padded.to(device=dev, dtype=torch.float32).contiguous()
+    assert audio.shape[0] == B and audio.shape[1] >= ((W - 1) * step + window) * spf, audio.shape
+    spk = engine.speaker_rows(speaker_id.to(dev))
+    frames = W * step + pre
+
+    # ---- hoisted audio phase: all W x B slices as one window-major batch at `window` rows ----
+    mem_face, kv = engine.audio_phase(audio, 0, step * spf, W, window * spf, window, limits=limits.wav)
+    mem_face = mem_face.view(W, B, window, engine.E)
+    # Zeroed (memset, no kernel): rows no window writes stay finite for the full-length argmax and decode.
+    acc = {}
+    for k in ("rec_", "cls_"):
+        for p in PARTS:
+            acc[k + p] = torch.empty(B, frames, 256, device=dev)
+            if acc[k + p].is_cuda:
+                _lib.call("pm_memset_async", acc[k + p].data_ptr(), 0, acc[k + p].numel() * 4, ops._stream())
+            else:
+                acc[k + p].zero_()
+    n_groups = max(1, min(int(_STATE.get("groups", 1)), B // 8)) if torch.cuda.is_available() else 1
+    bounds = [B * g // n_groups for g in range(n_groups + 1)]
+
+    def sl(x, g0, g1):
+        if isinstance(x, ops.Act):
+            pl = x.p
+            return ops.Act(None if x.f is None else x.f[g0:g1], None if pl is None else ops.Planes(pl.t[:, g0:g1], pl.rows, pl.ch, 0))
+        return x[g0:g1]
+
+    def run_lane(lane):
+        g0, g1 = bounds[lane], bounds[lane + 1]
+        nb = g1 - g0
+        spk_l = (spk[0][g0:g1], spk[1][g0:g1])
+        seed = None
+        for j in range(W):
+            lim = limits.window(j, g0, g1)
+            win_in = ops.window_input(None, None, seed, engine.mask_embedding, j * step, window, pre, nsplit=_ns(),
+                                      f32=_ns() == 0, shape=(nb, frames, ch), row_limit=lim[0])
+            out = engine.window(win_in, spk_l, mem_face[j][g0:g1], [sl(_window_of(k, j, B), g0, g1) for k in kv],
+                                dest={k: v[g0:g1, j * step:j * step + window] for k, v in acc.items()}, lane=lane,
+                                limits=lim)
+            if j + 1 < W:                     # seed for the next window; only clips whose window j is full continue
+                nd = min(window, seed_decode_frames(cfg, vq))
+                tail = {k: v[:, window - nd:] for k, v in out.items()}
+                idx = {p: ops.row_argmax(tail["cls_" + p]) for p in PARTS}
+                index, latent = select_inputs(cfg, tail, idx)
+                dec = vq.decode(index, latent, lane=lane)
+                seed = dec["all_motion4inference"][:, nd - pre:]
+
+    if n_groups == 1:
+        run_lane(0)
+    else:
+        if getattr(engine, "_fork_lanes", None) is None or engine._fork_lanes.n_side != n_groups - 1:
+            engine._fork_lanes = _Fork(n_groups - 1)
+        engine._fork_lanes.run([lambda lane=lane: run_lane(lane) for lane in range(n_groups)])
     return acc

@@ -69,10 +69,13 @@ def _bs_ld(t: torch.Tensor):
     return (t.stride(0) if t.shape[0] > 1 else t.shape[1] * t.stride(1)), t.stride(1)
 
 
-def tapgemm(a, w, bias, *, rows_out=None, stride=1, pad=0, act=ACT_NONE, slope=0.0, residual=None, out=None):
+def tapgemm(a, w, bias, *, rows_out=None, stride=1, pad=0, act=ACT_NONE, slope=0.0, residual=None, out=None,
+            row_limit=None):
     """out[b,l,:] = act(bias + sum_t A[b, l*stride+t-pad, :] @ W[t].T + residual[b,l,:]).
 
-    a: (batch, rows_in, cin); w: (taps, cout, cin) contiguous; returns (batch, rows_out, cout)."""
+    a: (batch, rows_in, cin); w: (taps, cout, cin) contiguous; returns (batch, rows_out, cout).
+    row_limit: optional int32 device tensor (batch,) - ragged batch: rows l >= row_limit[b] are written as 0
+    (a negative limit: clip b is not written)."""
     _chk(a), _chk(w)
     batch, rows_in, cin = a.shape
     taps, cout, cin_w = w.shape
@@ -97,21 +100,39 @@ def tapgemm(a, w, bias, *, rows_out=None, stride=1, pad=0, act=ACT_NONE, slope=0
         out_v = flat(out)
         res_v = flat(residual) if residual is not None else None
         batch_k, rows_in_k, rows_out_k = 1, batch * rows_in, batch * rows_out
+        rows_per_clip = rows_out
     else:
         out_v, res_v, batch_k, rows_in_k, rows_out_k = out, residual, batch, rows_in, rows_out
+        rows_per_clip = 0
     a_bs, lda = _bs_ld(a)
     o_bs, ldo = _bs_ld(out_v)
     r_bs, ldr = _bs_ld(res_v) if res_v is not None else (0, 0)
-    _call("pm_tapgemm_f32", a.data_ptr(), a_bs, lda, batch_k, rows_in_k, cin,
-          w.data_ptr(), _ptr(bias), taps, stride, pad, rows_out_k, cout,
-          _ptr(res_v), r_bs, ldr, act, float(slope), out_v.data_ptr(), o_bs, ldo, _stream())
+    if row_limit is None:
+        _call("pm_tapgemm_f32", a.data_ptr(), a_bs, lda, batch_k, rows_in_k, cin,
+              w.data_ptr(), _ptr(bias), taps, stride, pad, rows_out_k, cout,
+              _ptr(res_v), r_bs, ldr, act, float(slope), out_v.data_ptr(), o_bs, ldo, _stream())
+    else:
+        _chk_limit(row_limit, batch)
+        _call("pm_tapgemm_f32_rl", a.data_ptr(), a_bs, lda, batch_k, rows_in_k, cin,
+              w.data_ptr(), _ptr(bias), taps, stride, pad, rows_out_k, cout,
+              _ptr(res_v), r_bs, ldr, act, float(slope), out_v.data_ptr(), o_bs, ldo, row_limit.data_ptr(), rows_per_clip,
+              _stream())
     return out
 
 
-def wav_stem(audio, a_bs, a_ws, batch, windows, n_samples, w1, b1, wd, bd, *, stride, pad, slope, offset=0, nsplit=0):
+def _chk_limit(t, n):
+    """A per-clip limit table: int32 device tensor of at least n entries, read by the kernel."""
+    _chk(t, torch.int32)
+    assert t.dim() == 1 and t.is_contiguous() and t.numel() >= n, (t.shape, n)
+
+
+def wav_stem(audio, a_bs, a_ws, batch, windows, n_samples, w1, b1, wd, bd, *, stride, pad, slope, offset=0, nsplit=0,
+             n_valid=None):
     """First WavEncoder block's two convolutions on the raw waveform.  `audio` is the flat (bs, n)
     tensor; sequence (b, w) starts at element offset + b*a_bs + w*a_ws and is n_samples long.
-    Returns (y1, sc): y1 as fp32 tensor (nsplit 0) or as the operand Planes of the conv that follows."""
+    Returns (y1, sc): y1 as fp32 tensor (nsplit 0) or as the operand Planes of the conv that follows.
+    n_valid: optional int32 device tensor (windows*batch,), window-major - ragged batch: sequence w*batch + b holds only
+    n_valid samples (later ones read as 0) and the rows it does not yield are written as 0."""
     _chk(audio)
     cout, ks = w1.shape
     rows_out = (n_samples + 2 * pad - ks) // stride + 1
@@ -122,9 +143,15 @@ def wav_stem(audio, a_bs, a_ws, batch, windows, n_samples, w1, b1, wd, bd, *, st
     else:
         y1 = torch.empty_like(sc)
         y_ptr, pa = y1.data_ptr(), (0, 0, 0, 0)
-    _call("pm_wav_stem_f32", audio.data_ptr() + 4 * offset, a_bs, a_ws, batch, windows, n_samples,
-          w1.data_ptr(), b1.data_ptr(), wd.data_ptr(), bd.data_ptr(), cout, ks, stride, pad, rows_out,
-          float(slope), y_ptr, sc.data_ptr(), *pa, _stream())
+    if n_valid is None:
+        _call("pm_wav_stem_f32", audio.data_ptr() + 4 * offset, a_bs, a_ws, batch, windows, n_samples,
+              w1.data_ptr(), b1.data_ptr(), wd.data_ptr(), bd.data_ptr(), cout, ks, stride, pad, rows_out,
+              float(slope), y_ptr, sc.data_ptr(), *pa, _stream())
+    else:
+        _chk_limit(n_valid, batch * windows)
+        _call("pm_wav_stem_rl", audio.data_ptr() + 4 * offset, a_bs, a_ws, batch, windows, n_samples,
+              w1.data_ptr(), b1.data_ptr(), wd.data_ptr(), bd.data_ptr(), cout, ks, stride, pad, rows_out,
+              float(slope), y_ptr, sc.data_ptr(), *pa, n_valid.data_ptr(), _stream())
     return y1, sc
 
 
@@ -176,21 +203,30 @@ def add_layernorm(x, r, gamma, beta, eps=1e-5, nsplit=0, f32=True):
     return _result(out, pl, nsplit)
 
 
-def attention(q, k, v, batch, heads, tq, tk, head_dim, nsplit=0, f32=True):
-    """q: (batch*tq, >=heads*head_dim) view, k/v: (batch*tk, ...) views (column slices allowed)."""
+def attention(q, k, v, batch, heads, tq, tk, head_dim, nsplit=0, f32=True, q_len=None, k_len=None):
+    """q: (batch*tq, >=heads*head_dim) view, k/v: (batch*tk, ...) views (column slices allowed).
+    q_len / k_len: optional int32 device tensors (batch,) - ragged batch: keys >= k_len[b] get probability 0, query rows
+    >= q_len[b] (all rows when k_len[b] == 0) are written as 0.  Both or neither."""
     for t in (q, k, v):
         _chk(t)
     E = heads * head_dim
     out = torch.empty(batch * tq, E, device=q.device, dtype=torch.float32) if (f32 or not nsplit) else None
     pl = _new_planes(nsplit, (batch, tq), E, q.device) if nsplit else None
-    _call("pm_attention_f32", q.data_ptr(), q.stride(0), k.data_ptr(), k.stride(0), v.data_ptr(), v.stride(0),
-          _ptr(out), E, batch, heads, tq, tk, head_dim, *_pargs(pl), _stream())
+    if k_len is None:
+        _call("pm_attention_f32", q.data_ptr(), q.stride(0), k.data_ptr(), k.stride(0), v.data_ptr(), v.stride(0),
+              _ptr(out), E, batch, heads, tq, tk, head_dim, *_pargs(pl), _stream())
+    else:
+        _chk_limit(q_len, batch), _chk_limit(k_len, batch)
+        _call("pm_attention_f32_rl", q.data_ptr(), q.stride(0), k.data_ptr(), k.stride(0), v.data_ptr(), v.stride(0),
+              _ptr(out), E, batch, heads, tq, tk, head_dim, *_pargs(pl), q_len.data_ptr(), k_len.data_ptr(), _stream())
     return _result(out, pl, nsplit)
 
 
-def attention_tc(q, q_col0, k, k_col0, v, v_col0, batch, heads, tq, tk, head_dim, nsplit=2, f32=False):
+def attention_tc(q, q_col0, k, k_col0, v, v_col0, batch, heads, tq, tk, head_dim, nsplit=2, f32=False, q_len=None,
+                 k_len=None):
     """Attention on the tcgen05 tensor cores (fp16x3 engine).  q / k / v: two-plane fp16 Planes whose columns
-    [*_col0 + h*head_dim, ...) hold head h (the packed q|k|v or k|v projection output is passed as is)."""
+    [*_col0 + h*head_dim, ...) hold head h (the packed q|k|v or k|v projection output is passed as is).
+    q_len / k_len: per-clip counts as in attention()."""
     for pl, rows in ((q, tq), (k, tk), (v, tk)):
         assert pl.t.dtype == torch.float16 and pl.t.shape[0] == 2 and pl.t.shape[1] == batch and pl.rows == rows, \
             "attention_tc needs two-plane fp16 operands of (batch, rows, ch)"
@@ -198,11 +234,19 @@ def attention_tc(q, q_col0, k, k_col0, v, v_col0, batch, heads, tq, tk, head_dim
     dev = q.t.device
     out = torch.empty(batch * tq, E, device=dev, dtype=torch.float32) if (f32 or not nsplit) else None
     pl = _new_planes(nsplit, (batch, tq), E, dev, dtype=torch.float16) if nsplit else None
-    _call("pm_attention_tc",
-          q.t.data_ptr(), q.t.stride(0), q.t.stride(1), q.t.stride(2), q.ch, q_col0,
-          k.t.data_ptr(), k.t.stride(0), k.t.stride(1), k.t.stride(2), k.ch, k_col0,
-          v.t.data_ptr(), v.t.stride(0), v.t.stride(1), v.t.stride(2), v.ch, v_col0,
-          _ptr(out), E, batch, heads, tq, tk, head_dim, *_pargs(pl), _stream())
+    if k_len is None:
+        _call("pm_attention_tc",
+              q.t.data_ptr(), q.t.stride(0), q.t.stride(1), q.t.stride(2), q.ch, q_col0,
+              k.t.data_ptr(), k.t.stride(0), k.t.stride(1), k.t.stride(2), k.ch, k_col0,
+              v.t.data_ptr(), v.t.stride(0), v.t.stride(1), v.t.stride(2), v.ch, v_col0,
+              _ptr(out), E, batch, heads, tq, tk, head_dim, *_pargs(pl), _stream())
+    else:
+        _chk_limit(q_len, batch), _chk_limit(k_len, batch)
+        _call("pm_attention_tc_rl",
+              q.t.data_ptr(), q.t.stride(0), q.t.stride(1), q.t.stride(2), q.ch, q_col0,
+              k.t.data_ptr(), k.t.stride(0), k.t.stride(1), k.t.stride(2), k.ch, k_col0,
+              v.t.data_ptr(), v.t.stride(0), v.t.stride(1), v.t.stride(2), v.ch, v_col0,
+              _ptr(out), E, batch, heads, tq, tk, head_dim, *_pargs(pl), q_len.data_ptr(), k_len.data_ptr(), _stream())
     return _result(out, pl, nsplit)
 
 
@@ -227,9 +271,10 @@ def add2(a, b, nsplit=0, f32=True):
     return _result(out, pl, nsplit)
 
 
-def window_input(motion, mask, seed, mask_embedding, start, win_len, pre, nsplit=0, f32=True, shape=None):
+def window_input(motion, mask, seed, mask_embedding, start, win_len, pre, nsplit=0, f32=True, shape=None, row_limit=None):
     """motion / mask: (batch, total_len, ch) or None = inference()'s defaults (then `shape` = (batch, total_len, ch));
-    seed: (batch, pre, ch) view with dense rows (any clip stride), None when pre == 0."""
+    seed: (batch, pre, ch) view with dense rows (any clip stride), None when pre == 0.
+    row_limit: optional int32 device tensor (batch,) - ragged batch: rows >= row_limit[b] are written as 0."""
     batch, total_len, ch = motion.shape if motion is not None else shape
     for t in (motion, mask):
         if t is not None:
@@ -243,8 +288,13 @@ def window_input(motion, mask, seed, mask_embedding, start, win_len, pre, nsplit
     dev = mask_embedding.device
     out = torch.empty(batch, win_len, ch, device=dev, dtype=torch.float32) if (f32 or not nsplit) else None
     pl = _new_planes(nsplit, (batch, win_len), ch, dev) if nsplit else None
-    _call("pm_window_input_f32", _ptr(motion), _ptr(mask), _ptr(seed), mask_embedding.data_ptr(),
-          _ptr(out), batch, total_len, start, win_len, pre, ch, seed_bs, *_pargs(pl), _stream())
+    if row_limit is None:
+        _call("pm_window_input_f32", _ptr(motion), _ptr(mask), _ptr(seed), mask_embedding.data_ptr(),
+              _ptr(out), batch, total_len, start, win_len, pre, ch, seed_bs, *_pargs(pl), _stream())
+    else:
+        _chk_limit(row_limit, batch)
+        _call("pm_window_input_rl", _ptr(motion), _ptr(mask), _ptr(seed), mask_embedding.data_ptr(),
+              _ptr(out), batch, total_len, start, win_len, pre, ch, seed_bs, *_pargs(pl), row_limit.data_ptr(), _stream())
     return _result(out, pl, nsplit)
 
 
@@ -300,7 +350,9 @@ def zero_flag(device):
     return flag
 
 
-def gather_rows(codebook, index, nsplit=0, f32=True):
+def gather_rows(codebook, index, nsplit=0, f32=True, row_limit=None):
+    """row_limit: optional int32 device tensor (index.shape[0],) for a (clips, rows) index - ragged batch: rows
+    >= row_limit[clip] are written as 0."""
     _chk(codebook), _chk(index, torch.int64)
     assert index.is_contiguous()
     ch = codebook.shape[1]
@@ -309,8 +361,14 @@ def gather_rows(codebook, index, nsplit=0, f32=True):
     if nsplit:
         lead = (index.shape[0], index.numel() // index.shape[0]) if index.dim() > 1 else (1, index.numel())
         pl = _new_planes(nsplit, lead, ch, codebook.device)
-    _call("pm_gather_rows_f32", codebook.data_ptr(), codebook.shape[0], index.data_ptr(), index.numel(), ch, _ptr(out),
-          *_pargs(pl), _stream())
+    if row_limit is None:
+        _call("pm_gather_rows_f32", codebook.data_ptr(), codebook.shape[0], index.data_ptr(), index.numel(), ch, _ptr(out),
+              *_pargs(pl), _stream())
+    else:
+        assert index.dim() == 2
+        _chk_limit(row_limit, index.shape[0])
+        _call("pm_gather_rows_rl", codebook.data_ptr(), codebook.shape[0], index.data_ptr(), index.numel(), ch, _ptr(out),
+              *_pargs(pl), row_limit.data_ptr(), index.shape[1], _stream())
     return _result(out, pl, nsplit)
 
 
@@ -421,10 +479,13 @@ class PackedW:
 
 
 def tapgemm_tc(a: Planes, w: PackedW, bias, *, rows_in=None, rows_out, pad=0, act=ACT_NONE, act_cols=0, slope=0.0,
-               residual=None, want_f32=True, out_nsplit=0, out=None, a_view=None, out_slack=0, prefetch=None):
+               residual=None, want_f32=True, out_nsplit=0, out=None, a_view=None, out_slack=0, prefetch=None,
+               row_limit=None, rows_per_clip=0):
     """Tensor-core tap-GEMM.  `prefetch`: a tensor (the next GEMM's packed weights) to pull into L2 meanwhile.
     `a_view` = (rows_in, cin, lda) overrides the logical view of the A planes
-    (strided convs pass the (rows/s, s*C) view of the same memory).  Returns (fp32 out | None, Planes | None)."""
+    (strided convs pass the (rows/s, s*C) view of the same memory).  Returns (fp32 out | None, Planes | None).
+    row_limit: optional int32 device tensor of per-clip valid output rows (ragged batch; include/pm_emage.h
+    pm_tapgemm_tc_rl); the clip is the batch index, or row // rows_per_clip of a flat (1, clips*rows) launch."""
     t = a.t
     nsplit, batch = t.shape[0], t.shape[1]
     assert nsplit == w.t.shape[0] and t.dtype == w.t.dtype, "A and W must use the same split and plane format"
@@ -447,15 +508,21 @@ def tapgemm_tc(a: Planes, w: PackedW, bias, *, rows_in=None, rows_out, pad=0, ac
     if residual is not None:
         _chk(residual)
         assert residual.shape == (batch, rows_out, cout)
-    _call("pm_tapgemm_tc", t.data_ptr(), t.stride(0), t.stride(1), lda, batch, rows_a, cin,
-          w.t.data_ptr(), w.t.stride(0), w.w_rows, w.ldw, w.taps, pad, nsplit | fmt,
-          _ptr(bias), rows_out, cout, _ptr(residual), r_bs, ldr, act, act_cols, float(slope), float(w.acc_scale),
-          _ptr(out_f), o_bs, ldo,
-          None if out_p is None else out_p.t.data_ptr(), 0 if out_p is None else out_p.t.stride(0),
-          0 if out_p is None else out_p.t.stride(1), 0 if out_p is None else out_p.t.stride(2),
-          out_nsplit | (fmt if out_nsplit else 0),
-          None if prefetch is None else prefetch.data_ptr(),
-          0 if prefetch is None else prefetch.numel() * prefetch.element_size(), _stream())
+    ob = (None, 0, 0, 0) if out_p is None else (out_p.t.data_ptr(), out_p.t.stride(0), out_p.t.stride(1), out_p.t.stride(2))
+    pf_ptr, pf_bytes = (None, 0) if prefetch is None else (prefetch.data_ptr(), prefetch.numel() * prefetch.element_size())
+    if row_limit is None:
+        _call("pm_tapgemm_tc", t.data_ptr(), t.stride(0), t.stride(1), lda, batch, rows_a, cin,
+              w.t.data_ptr(), w.t.stride(0), w.w_rows, w.ldw, w.taps, pad, nsplit | fmt,
+              _ptr(bias), rows_out, cout, _ptr(residual), r_bs, ldr, act, act_cols, float(slope), float(w.acc_scale),
+              _ptr(out_f), o_bs, ldo, ob[0], ob[1], ob[2], ob[3], out_nsplit | (fmt if out_nsplit else 0),
+              pf_ptr, pf_bytes, _stream())
+    else:
+        _chk_limit(row_limit, -(-batch * rows_out // rows_per_clip) if rows_per_clip else batch)
+        _call("pm_tapgemm_tc_rl", t.data_ptr(), t.stride(0), t.stride(1), lda, batch, rows_a, cin,
+              w.t.data_ptr(), w.t.stride(0), w.w_rows, w.ldw, w.taps, pad, nsplit | fmt,
+              _ptr(bias), rows_out, cout, _ptr(residual), r_bs, ldr, act, act_cols, float(slope), float(w.acc_scale),
+              _ptr(out_f), o_bs, ldo, ob[0], ob[1], ob[2], ob[3], out_nsplit | (fmt if out_nsplit else 0),
+              pf_ptr, pf_bytes, row_limit.data_ptr(), rows_per_clip, _stream())
     return out_f, out_p
 
 
